@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark: complex IQ GS/s of persistence_spectrum on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[2], the configuration the metric is quoted on): persistence
 spectrum of 100 MS/s complex64 captures, 10 s per channel (1e9 samples), nfft 4096 Hann, 50 %
@@ -297,6 +297,16 @@ def extra_configs(torch, iqw, dev, peak):
     return rows
 
 
+def dump_outputs(out_dir, arrays):
+    """what the last timed step returned, one float32 `<name>.npy` per array: the inputs are regenerated from fixed
+    seeds, so two builds run with the same arguments can be compared output for output"""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), t.float().cpu().numpy())
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -349,10 +359,16 @@ def run_b200(args):
     barrier()
     e0.record()
     for _ in range(args.steps):
-        step(x)
+        out = step(x)
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump = {'persistence_spectrum': out}
+        if world > 1:
+            dump['gathered_rows'] = gathered['rows']
+        dump_outputs(args.dump_outputs, dump)
+    del out
     prof = _lib.profile_report()
     _lib.profile(False)
     clocks = sampler.stop() if sampler else None
@@ -519,7 +535,15 @@ def main():
     ap.add_argument('--no-e2e', action='store_true')
     ap.add_argument('--no-cpu', action='store_true')
     ap.add_argument('--no-extra', action='store_true', help='skip the one-shot timings of the other configs')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the result of the last timed step as DIR/persistence_spectrum.npy (float32, '
+                         '4 quantile rows x 4096 bins per channel) and, on more than one GPU, the all-gathered rows '
+                         'of every channel as DIR/gathered_rows.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs writes the outputs of the GPU path (--impl b200)')
     if args.impl == 'reference':
         with QuietStdout():
             line = run_reference(args)

@@ -37,13 +37,16 @@ def test_ola_filter_golden(name):
 @pytest.mark.parametrize('nfft', [16, 32, 64, 128, 256, 512, 1024, 2048, 4096, 8192])
 @pytest.mark.parametrize('R', [1, 2, 4, 8, 16])
 def test_istft_matches_oracle(nfft, R):
-    if R > (8 if nfft in (32, 64) else 16):
-        pytest.skip('nfft/hop larger than the values a thread holds')
     hop = nfft // R
     T = 37
     x = synth(nfft + R, (2, (T - 1) * hop + nfft))
     y = orc.stft(x, fs=1e6, window='hamming', nperseg=nfft, noverlap=nfft - hop, axis=1, truncate=False,
                  return_axis_arrays=False)
+    if R > (8 if nfft in (32, 64) else 16):
+        # nfft/hop larger than the values a thread holds: the library refuses the geometry
+        with pytest.raises(NotImplementedError):
+            iqw.istft(torch.from_numpy(y).cuda(), nfft=nfft, noverlap=nfft - hop, axis=1)
+        return
     want = orc.istft(y.copy(), None, nfft=nfft, noverlap=nfft - hop, axis=1)
     got = iqw.istft(torch.from_numpy(y).cuda(), nfft=nfft, noverlap=nfft - hop, axis=1)
     _check(got.cpu().numpy(), want)

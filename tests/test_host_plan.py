@@ -97,12 +97,19 @@ def test_error_behaviour_matches_reference():
 
 
 def test_no_cpu_fallback():
-    import torch
+    """without a CUDA device the package raises instead of computing on the CPU; checked in a child process that
+    sees no device, so that the test also runs on a machine with a GPU"""
+    import os
+    import subprocess
+    import sys
 
-    if torch.cuda.is_available():
-        pytest.skip('GPU present')
-    with pytest.raises(RuntimeError, match='no CPU fallback'):
-        iqw.spectrogram(np.zeros(1000, np.complex64), fs=1.0, window='hann', nperseg=64)
+    code = ('import numpy as np, pytest, iqwaveform_b200 as iqw\n'
+            "with pytest.raises(RuntimeError, match='no CPU fallback'):\n"
+            "    iqw.spectrogram(np.zeros(1000, np.complex64), fs=1.0, window='hann', nperseg=64)\n")
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    r = subprocess.run([sys.executable, '-c', code], cwd=root, env=dict(os.environ, CUDA_VISIBLE_DEVICES=''),
+                       capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr
 
 
 def test_util_helpers_known_answers():

@@ -12,6 +12,14 @@ SPG = ['spg_bh_2048_1024', 'spg_hann_1024_768', 'spg_rect_4096_0']
 PSD = ['psd_hann_1024_half', 'psd_hann_4096_trim', 'psd_bh_256_linear']
 
 
+@pytest.fixture(autouse=True)
+def _fixture_fft_threads(monkeypatch):
+    """the reference runs its FFTs on os.cpu_count() // 2 threads, and the thread count changes the last bits of some
+    transforms: the oracle uses the CPU count of the machine that wrote the fixtures (8; only then does
+    spg_bh_2048_1024 match), whatever machine runs the test"""
+    monkeypatch.setattr(orc, 'CPU_COUNT', 8)
+
+
 @pytest.mark.parametrize('name', STFT)
 def test_stft_bitwise(name):
     p, a = load_golden(name)
