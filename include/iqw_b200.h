@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define IQW_ABI_VERSION 8
+#define IQW_ABI_VERSION 9
 
 typedef enum iqw_status {
     IQW_OK = 0,
@@ -255,6 +255,30 @@ int iqw_ola_filter_c64(const void* d_x, int64_t n_channels, int64_t n_samples, i
  */
 int iqw_edge_counts_f32(const float* d_a, int64_t n_rows, int64_t n_cols, const double* d_edges,
                         int32_t n_edges, int32_t side_right, int64_t* d_counts, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Kernel 6: polyphase FIR filter / rational resampler with the semantics of scipy.signal.upfirdn
+ * (zero padding only): zero-stuff by `up`, convolve in full with the L taps h, keep every `down`-th
+ * sample.  Replaces the reference's fourier.upfirdn (fourier.py:1476-1495: scipy.signal.upfirdn on
+ * the host, the NVRTC polyphase kernel of cuda.py on cupy arrays).
+ *
+ *   y[n] = sum_{j < Lp} hp[p][j] * x[i0 - j],  t = n*down, p = t mod up, i0 = t div up
+ *
+ *   d_x           (n_channels, n_in) complex64, row stride x_channel_stride elements; d_x[0] is the
+ *                 sample of GLOBAL index x_first (0 for a whole capture; a time shard passes the first
+ *                 sample it holds).  Samples outside [x_first, x_first + n_in) read as zero
+ *   d_taps        the polyphase table hp[p][j] = h[p + j*up] for p < min(up, n_taps) and
+ *                 j < Lp = ceil(n_taps/up), zero-padded: float32 (taps_complex = 0) or complex64
+ *                 (python: iqwaveform_b200._plan.upfirdn_polyphase).  At most 32768 floats
+ *                 (16384 real or 8192 complex taps for any up; larger: IQW_ERR_UNSUPPORTED)
+ *   out_first     global index of the first output; the call writes outputs
+ *                 [out_first, out_first + n_out) to d_out (n_channels, n_out) complex64, channel stride
+ *                 out_channel_stride elements
+ * The summation order of an output depends only on its global index and (up, down, n_taps), so shards
+ * of one capture concatenate to the bits of a single call. */
+int iqw_upfirdn_c64(const void* d_x, int64_t n_channels, int64_t n_in, int64_t x_channel_stride, int64_t x_first,
+                    const void* d_taps, int32_t taps_complex, int32_t n_taps, int32_t up, int32_t down,
+                    int64_t out_first, int64_t n_out, void* d_out, int64_t out_channel_stride, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Exact order statistics of a float32 matrix whose ROWS are spread over several GPUs (the

@@ -299,3 +299,31 @@ def split_requests(reqs, n_rows: int):
     if cur:
         groups.append(cur)
     return groups
+
+
+# polyphase table limit of iqw_upfirdn_c64: 16384 real or 8192 complex taps for any up
+UPFIRDN_MAX_TABLE_FLOATS = 32768
+
+
+def upfirdn_output_len(n_taps: int, n_in: int, up: int, down: int) -> int:
+    """output length of scipy.signal.upfirdn (scipy's _output_len): the full convolution of the
+    zero-stuffed input, (n_in - 1)*up + n_taps samples, kept every `down`-th, rounded up"""
+    if n_in < 1:
+        return 0
+    return ((n_in - 1) * up + n_taps - 1) // down + 1
+
+
+def upfirdn_polyphase(h: np.ndarray, up: int) -> np.ndarray:
+    """polyphase table hp[p][j] = h[p + j*up], p < min(up, len(h)), j < ceil(len(h)/up), zero-padded.
+    Rows p >= len(h) would be all zero and are left out (the kernel treats them as zero)."""
+    L = h.shape[0]
+    lp = -(-L // up)
+    padded = np.zeros(lp * up, dtype=h.dtype)
+    padded[:L] = h
+    return np.ascontiguousarray(padded.reshape(lp, up).T[:min(up, L)])
+
+
+def upfirdn_phase_index(n: np.ndarray, up: int, down: int) -> tuple[np.ndarray, np.ndarray]:
+    """(p, i0) of global output indices n: y[n] = sum_j hp[p][j] * x[i0 - j]"""
+    t = np.asarray(n, dtype=np.int64) * down
+    return t % up, t // up

@@ -9,6 +9,8 @@ The path shards without any collective on the data path, with one exception (the
   `noverlap` samples are the halo shared with the next rank
 * power bins are independent                   -> `bin_shard`      (iq_to_bin_power, config 4):
   shards are aligned to whole bins, so the halo is zero
+* upfirdn outputs are independent              -> `upfirdn_shard`  (upfirdn): rank r owns outputs
+  [out0, out1) and reads the Lp - 1 samples before its first input as the halo
 * exact quantiles of ONE capture split in time -> `persistence_spectrum_time_sharded`: the only
   real exchange step of the path -- per-bin digit counts of a radix select are all_reduced
   (`select_order_statistics`; kernels in csrc/iqw_rowsplit.cu)
@@ -25,7 +27,8 @@ import torch.distributed as dist
 
 __all__ = ['channel_shard', 'frame_shard', 'bin_shard', 'gather_rows', 'persistence_spectrum_sharded',
            'persistence_spectrum_time_sharded', 'select_order_statistics', 'CudaShardOps', 'ThreadGroup',
-           'bind_to_gpu_numa_node', 'spectrogram_time_sharded', 'iq_to_bin_power_sharded']
+           'bind_to_gpu_numa_node', 'spectrogram_time_sharded', 'iq_to_bin_power_sharded', 'upfirdn_shard',
+           'upfirdn_time_sharded']
 
 
 def _split(n: int, world: int, rank: int) -> tuple[int, int]:
@@ -516,3 +519,58 @@ def iq_to_bin_power_sharded(x_local, Ts: float, Tbin: float, *, n_samples: int, 
         return out
     sizes = [(lambda s: s.bin1 - s.bin0)(bin_shard(n_samples, bin_len, world, r)) for r in range(world)]
     return gather_rows(out, sizes, 0, group)
+
+
+class UpfirdnShard(NamedTuple):
+    out0: int       # first output of this rank
+    out1: int       # one past its last output
+    sample0: int    # first sample it reads
+    sample1: int    # one past the last sample it reads (includes the halo)
+    n_out: int      # outputs of the whole capture
+
+
+def upfirdn_shard(n_in: int, n_taps: int, up: int, down: int, world: int, rank: int) -> UpfirdnShard:
+    """time-axis shard of upfirdn: outputs split evenly; the samples are those the rank's outputs read,
+    y[n] = sum_{j < Lp} hp[p][j] * x[n*down div up - j], clamped to [0, n_in)"""
+    from . import _plan
+    if n_taps < 1 or up < 1 or down < 1:
+        raise ValueError('need n_taps, up, down >= 1')
+    n_out = _plan.upfirdn_output_len(n_taps, n_in, up, down)
+    o0, o1 = _split(n_out, world, rank)
+    lp = -(-n_taps // up)
+    if o1 == o0:
+        s = min(o0 * down // up, n_in)
+        return UpfirdnShard(o0, o1, s, s, n_out)
+    s0 = max(0, o0 * down // up - (lp - 1))
+    s1 = min(n_in, (o1 - 1) * down // up + 1)
+    return UpfirdnShard(o0, o1, s0, max(s0, s1), n_out)
+
+
+def upfirdn_time_sharded(x_halo, h, up: int = 1, down: int = 1, *, n_samples: int, group=None,
+                         compute: Callable | None = None, gather: bool = False):
+    """time-sharded upfirdn of a 1-D complex64 capture of `n_samples` samples: `x_halo` holds this rank's
+    samples [shard.sample0, shard.sample1) of `upfirdn_shard` (halo included).  Returns this rank's
+    outputs [out0, out1) or, with gather=True, all outputs on every rank; the concatenation is bitwise
+    the single-GPU `upfirdn`.  `compute(x_halo, table, n_taps, up, down, x_first=, out_first=, n_out=)`
+    defaults to the CUDA kernel."""
+    from . import fourier
+    up, down = int(up), int(down)
+    table, n_taps = fourier._upfirdn_taps(h, up, down)
+    world, rank = _world(group)
+    sh = upfirdn_shard(n_samples, n_taps, up, down, world, rank)
+    if x_halo.ndim != 1 or x_halo.shape[0] != sh.sample1 - sh.sample0:
+        raise ValueError(f'rank {rank} expects a 1-D shard of {sh.sample1 - sh.sample0} samples, got {tuple(x_halo.shape)}')
+    if compute is None:
+        from . import _arrays
+        xd, _ = _arrays.to_device(x_halo)
+        if xd.dtype != torch.complex64:
+            raise NotImplementedError(f'upfirdn: only complex64 x is built (got {xd.dtype})')
+        y = fourier._upfirdn_device(xd.reshape(1, -1), table, n_taps, up, down, x_first=sh.sample0,
+                                    out_first=sh.out0, n_out=sh.out1 - sh.out0)[0]
+    else:
+        y = torch.as_tensor(compute(x_halo, table, n_taps, up, down, x_first=sh.sample0, out_first=sh.out0,
+                                    n_out=sh.out1 - sh.out0))
+    if not gather or world == 1:
+        return y
+    sizes = [(lambda s: s.out1 - s.out0)(upfirdn_shard(n_samples, n_taps, up, down, world, r)) for r in range(world)]
+    return gather_rows(y, sizes, 0, group)

@@ -26,7 +26,7 @@ from . import _arrays, _lib, _plan
 from .util import Domain, get_input_domain
 from ._plan import INF
 
-__all__ = ['GraphedCall', 'fft', 'ifft', 'zero_stft_by_freq', 'stft', 'istft', 'ola_filter', 'oaresample', 'iq_to_stft_spectrogram', 'channelize_power', 'spectrogram', 'power_spectral_density', 'persistence_spectrum',
+__all__ = ['GraphedCall', 'fft', 'ifft', 'zero_stft_by_freq', 'stft', 'istft', 'ola_filter', 'oaresample', 'upfirdn', 'iq_to_stft_spectrogram', 'channelize_power', 'spectrogram', 'power_spectral_density', 'persistence_spectrum',
            'fftfreq', 'get_window', 'equivalent_noise_bandwidth']
 
 fftfreq = _plan.fftfreq
@@ -524,6 +524,74 @@ def oaresample(x, up, down, fs, *, window='hamming', overwrite_x=False, axis=1, 
     xr = _istft_device(y, nfft_out, noverlap, bin_lo=place_lo, bin_hi=place_hi, gain=gain,
                        scale=float(np.float32(factor)))
     return res.give_back(_arrays.restore_layout(xr, lead, trail, 1))
+
+
+_UPFIRDN_MODES = ('constant', 'wrap', 'edge', 'smooth', 'symmetric', 'reflect', 'antisymmetric', 'antireflect',
+                  'line')
+
+
+def _upfirdn_taps(h, up: int, down: int, mode='constant', cval=0) -> tuple[np.ndarray, int]:
+    """scipy.signal.upfirdn's argument checks (ValueError) and what is not built here
+    (NotImplementedError), all on the host; returns (polyphase table float32 | complex64, len(h))"""
+    if isinstance(h, torch.Tensor):
+        h = h.detach().cpu().numpy()
+    h = np.asarray(h)
+    if h.ndim != 1 or h.size == 0:
+        raise ValueError('h must be 1-D with non-zero length')
+    if up < 1 or down < 1:
+        raise ValueError('Both up and down must be >= 1')
+    if mode not in _UPFIRDN_MODES:
+        raise ValueError(f'Unknown mode: {mode!r}')
+    if mode != 'constant' or cval != 0:
+        raise NotImplementedError("upfirdn: only mode='constant' with cval=0 (zero padding) is built")
+    h = h.astype(np.complex64 if np.iscomplexobj(h) else np.float32)
+    table = _plan.upfirdn_polyphase(h, up)
+    if table.size * (2 if table.dtype == np.complex64 else 1) > _plan.UPFIRDN_MAX_TABLE_FLOATS:
+        raise NotImplementedError(f'upfirdn: a polyphase table of {table.shape[0]} x {table.shape[1]} taps exceeds '
+                                  f'{_plan.UPFIRDN_MAX_TABLE_FLOATS} floats (16384 real or 8192 complex taps)')
+    return table, h.size
+
+
+def _upfirdn_device(x2: torch.Tensor, table: np.ndarray, n_taps: int, up: int, down: int, *, x_first: int = 0,
+                    out_first: int = 0, n_out: int) -> torch.Tensor:
+    """(C, N) complex64 device rows holding global samples [x_first, x_first + N) -> (C, n_out) outputs
+    [out_first, out_first + n_out) of the whole capture.  The kernel reads unit-stride rows: any other
+    layout (a column of an (N, C) capture, a strided view) is copied first."""
+    C, N = x2.shape
+    if x2.stride(1) != 1 or (C > 1 and x2.stride(0) < N):
+        x2 = x2.contiguous()
+    y = torch.empty((C, n_out), dtype=torch.complex64, device=x2.device)
+    if n_out == 0 or C == 0:
+        return y
+    taps = torch.from_numpy(table).to(x2.device)
+    _lib.check(_lib.lib.iqw_upfirdn_c64(
+        ctypes.c_void_p(x2.data_ptr()), C, N, x2.stride(0) if C > 1 else N, x_first, ctypes.c_void_p(taps.data_ptr()),
+        int(table.dtype == np.complex64), n_taps, up, down, out_first, n_out, ctypes.c_void_p(y.data_ptr()), n_out,
+        _stream_ptr(x2.device)))
+    return y
+
+
+def upfirdn(h, x, up=1, down=1, axis=-1, mode='constant', cval=0):
+    """upsample by `up` (zero stuffing), FIR-filter with `h` in full, downsample by `down`, along `axis`;
+    the arguments and output length of scipy.signal.upfirdn, which the reference forwards host arrays to
+    (fourier.py:1476-1495).  Polyphase: only the taps that meet a non-zero sample are applied.
+
+    Differences from scipy: the arithmetic is float32.  `h` (1-D, real or complex, any float dtype) is
+    rounded once to float32 / complex64, and the result is always complex64 -- scipy returns
+    complex128 for float64 taps.  `x` must be complex64.  Only zero padding is built (mode='constant',
+    cval=0; other modes raise NotImplementedError, unknown ones ValueError), as in the reference's GPU
+    path, and the polyphase table is limited to 32768 floats: 16384 real or 8192 complex taps, for any
+    `up`."""
+    up, down = int(up), int(down)
+    table, n_taps = _upfirdn_taps(h, up, down, mode, cval)
+    dtype = getattr(x, 'dtype', None)
+    if dtype not in (np.complex64, torch.complex64):
+        raise NotImplementedError(f'upfirdn: only complex64 x is built (got {dtype})')
+    xd, res = _arrays.to_device(x)
+    x2, lead, trail = _arrays.as_channels(xd, axis)
+    n_out = _plan.upfirdn_output_len(n_taps, x2.shape[1], up, down)
+    y = _upfirdn_device(x2, table, n_taps, up, down, n_out=n_out)
+    return res.give_back(_arrays.restore_layout(y, lead, trail, 1))
 
 
 def _python_slice(n: int, start: int, stop_from_end: int) -> tuple[int, int]:
