@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define IQW_ABI_VERSION 9
+#define IQW_ABI_VERSION 10
 
 typedef enum iqw_status {
     IQW_OK = 0,
@@ -279,6 +279,34 @@ int iqw_edge_counts_f32(const float* d_a, int64_t n_rows, int64_t n_cols, const 
 int iqw_upfirdn_c64(const void* d_x, int64_t n_channels, int64_t n_in, int64_t x_channel_stride, int64_t x_first,
                     const void* d_taps, int32_t taps_complex, int32_t n_taps, int32_t up, int32_t down,
                     int64_t out_first, int64_t n_out, void* d_out, int64_t out_channel_stride, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Kernel 7: FFT convolution of complex64 rows with an M-tap filter by overlap-save, the output windows
+ * of scipy.signal.oaconvolve.  Replaces the reference's fourier.oaconvolve (fourier.py:1496-1509:
+ * scipy.signal.oaconvolve on the host, cupyx on cupy arrays).
+ *
+ *   y[n] = sum_{k < n_taps} h[k] * x[n - k],  n a global index of the full convolution
+ *
+ *   d_x           (n_channels, n_in) complex64, row stride x_channel_stride elements; d_x[0] is the
+ *                 sample of GLOBAL index x_first (0 for a whole capture; a time shard passes the first
+ *                 sample it holds).  Samples outside [x_first, x_first + n_in) read as zero
+ *   d_hspec       H = fft(h, nfft) / nfft, complex64, one row (hspec_channel_stride = 0: the same
+ *                 filter for every channel) or one row per channel (hspec_channel_stride = nfft)
+ *                 (python: iqwaveform_b200._plan.oaconvolve_spectrum)
+ *   nfft, discard blocks of nfft samples keep their last nfft - discard; nfft/discard in {2, 4, 8, 16},
+ *                 discard >= n_taps - 1 (else IQW_ERR_INVALID).  Built: the (nfft, discard) pairs
+ *                 that python's _plan.oaconvolve_plan picks for 1..4097 taps; other pairs return
+ *                 IQW_ERR_UNSUPPORTED
+ *   out_first     global index of the first output; the call writes outputs
+ *                 [out_first, out_first + n_out) to d_out (n_channels, n_out) complex64, channel stride
+ *                 out_channel_stride elements
+ * Blocks are anchored at global index 0, never at out_first: a window of the full convolution is a
+ * bitwise crop of it, and time shards that hold each of their blocks' in-range samples (the discard
+ * before their first output) concatenate to the bits of a single call. */
+int iqw_oaconvolve_c64(const void* d_x, int64_t n_channels, int64_t n_in, int64_t x_channel_stride, int64_t x_first,
+                       const void* d_hspec, int64_t hspec_channel_stride, int32_t n_taps, int32_t nfft,
+                       int32_t discard, int64_t out_first, int64_t n_out, void* d_out, int64_t out_channel_stride,
+                       void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Exact order statistics of a float32 matrix whose ROWS are spread over several GPUs (the

@@ -327,3 +327,49 @@ def upfirdn_phase_index(n: np.ndarray, up: int, down: int) -> tuple[np.ndarray, 
     """(p, i0) of global output indices n: y[n] = sum_j hp[p][j] * x[i0 - j]"""
     t = np.asarray(n, dtype=np.int64) * down
     return t % up, t // up
+
+
+# filters longer than this would need nfft > 8192 (discard nfft/2 >= M - 1): not built
+OACONVOLVE_MAX_TAPS = 4097
+
+
+@functools.lru_cache(maxsize=None)
+def oaconvolve_plan(n_taps: int) -> tuple[int, int]:
+    """(nfft, discard) of the overlap-save blocks of iqw_oaconvolve_c64 for an M-tap filter: nfft a
+    power of two in 16..8192, discard D = nfft/R with R in {2, 4, 8, 16} and D >= M - 1, hop = nfft - D.
+    Minimises the transform work per output, log2(nfft) * nfft / hop (exactly: log2(nfft) * R / (R - 1));
+    a tie goes to the smaller nfft."""
+    from fractions import Fraction
+    if not 1 <= n_taps <= OACONVOLVE_MAX_TAPS:
+        raise ValueError(f'oaconvolve plan: need 1 <= n_taps <= {OACONVOLVE_MAX_TAPS} (got {n_taps})')
+    best = None
+    for log2n in range(4, 14):
+        for r in (2, 4, 8, 16):
+            nfft = 1 << log2n
+            if nfft // r < n_taps - 1:
+                continue
+            cost = Fraction(log2n * r, r - 1)
+            if best is None or cost < best[0]:
+                best = (cost, nfft, nfft // r)
+    return best[1], best[2]
+
+
+def oaconvolve_window(mode: str, n1: int, n2: int) -> tuple[int, int]:
+    """(first, length) of the output of scipy.signal.oaconvolve along the convolved axis, as a window
+    of the full convolution (length n1 + n2 - 1); n1 is the length of in1 along that axis"""
+    L = n1 + n2 - 1
+    if mode == 'full':
+        return 0, L
+    if mode == 'same':
+        return (L - n1) // 2, n1
+    if mode == 'valid':
+        return min(n1, n2) - 1, max(n1, n2) - min(n1, n2) + 1
+    raise ValueError("acceptable mode flags are 'valid', 'same', or 'full'")
+
+
+def oaconvolve_spectrum(h: np.ndarray, nfft: int) -> np.ndarray:
+    """H = fft(h, nfft) / nfft along the last axis, computed in float64 and rounded once to complex64
+    (the 1/nfft of the inverse transform is folded in)"""
+    h = np.asarray(h)
+    H = np.fft.fft(h.astype(np.complex128), nfft, axis=-1) / nfft
+    return np.ascontiguousarray(H.astype(np.complex64))

@@ -11,6 +11,9 @@ The path shards without any collective on the data path, with one exception (the
   shards are aligned to whole bins, so the halo is zero
 * upfirdn outputs are independent              -> `upfirdn_shard`  (upfirdn): rank r owns outputs
   [out0, out1) and reads the Lp - 1 samples before its first input as the halo
+* oaconvolve outputs are independent           -> `oaconvolve_shard` (oaconvolve): rank r owns outputs
+  [out0, out1) and reads every in-range sample of the overlap-save blocks they fall in -- a halo of
+  the discard D (not M - 1) before them and the rest of its last block after them
 * exact quantiles of ONE capture split in time -> `persistence_spectrum_time_sharded`: the only
   real exchange step of the path -- per-bin digit counts of a radix select are all_reduced
   (`select_order_statistics`; kernels in csrc/iqw_rowsplit.cu)
@@ -22,13 +25,14 @@ from __future__ import annotations
 
 from typing import Callable, NamedTuple
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
 __all__ = ['channel_shard', 'frame_shard', 'bin_shard', 'gather_rows', 'persistence_spectrum_sharded',
            'persistence_spectrum_time_sharded', 'select_order_statistics', 'CudaShardOps', 'ThreadGroup',
            'bind_to_gpu_numa_node', 'spectrogram_time_sharded', 'iq_to_bin_power_sharded', 'upfirdn_shard',
-           'upfirdn_time_sharded']
+           'upfirdn_time_sharded', 'oaconvolve_shard', 'oaconvolve_time_sharded']
 
 
 def _split(n: int, world: int, rank: int) -> tuple[int, int]:
@@ -573,4 +577,70 @@ def upfirdn_time_sharded(x_halo, h, up: int = 1, down: int = 1, *, n_samples: in
     if not gather or world == 1:
         return y
     sizes = [(lambda s: s.out1 - s.out0)(upfirdn_shard(n_samples, n_taps, up, down, world, r)) for r in range(world)]
+    return gather_rows(y, sizes, 0, group)
+
+
+class OaconvolveShard(NamedTuple):
+    out0: int       # first output of this rank (index into the output of the chosen mode)
+    out1: int       # one past its last output
+    sample0: int    # first sample it reads
+    sample1: int    # one past the last sample it reads (includes the halo)
+    n_out: int      # outputs of the whole capture in the chosen mode
+
+
+def oaconvolve_shard(n_in: int, n_taps: int, mode: str, world: int, rank: int) -> OaconvolveShard:
+    """time-axis shard of oaconvolve(x, h, mode) for a capture of n_in samples and an n_taps filter:
+    the outputs of the mode are split evenly; the samples are every in-range sample of the overlap-save
+    blocks those outputs fall in (block b reads [b*hop - D, b*hop - D + nfft)), clamped to [0, n_in).
+    Every block is then computed from the same samples as in one call, so the shards' concatenation is
+    bitwise the single-GPU result."""
+    from . import _plan
+    if n_taps < 1 or n_in < n_taps:
+        raise NotImplementedError(f'oaconvolve time shards need 1 <= n_taps <= n_in (got {n_taps}, {n_in})')
+    nfft, discard = _plan.oaconvolve_plan(n_taps)
+    hop = nfft - discard
+    first, n_out = _plan.oaconvolve_window(mode, n_in, n_taps)
+    o0, o1 = _split(n_out, world, rank)
+    if o1 == o0:
+        s = min(max(0, (first + o0) // hop * hop - discard), n_in)
+        return OaconvolveShard(o0, o1, s, s, n_out)
+    b0, b1 = (first + o0) // hop, (first + o1 - 1) // hop
+    s0 = min(n_in, max(0, b0 * hop - discard))
+    s1 = min(n_in, b1 * hop - discard + nfft)
+    return OaconvolveShard(o0, o1, s0, max(s0, s1), n_out)
+
+
+def oaconvolve_time_sharded(x_halo, h, mode: str = 'full', *, n_samples: int, group=None,
+                            compute: Callable | None = None, gather: bool = False):
+    """time-sharded oaconvolve(x, h, mode) of a 1-D complex64 capture x of `n_samples` samples and a 1-D
+    filter h no longer than it: `x_halo` holds this rank's samples [shard.sample0, shard.sample1) of
+    `oaconvolve_shard` (halo included).  Returns this rank's outputs [out0, out1) or, with gather=True, all
+    outputs on every rank; the concatenation is bitwise the single-GPU `oaconvolve`.
+    `compute(x_halo, hspec, n_taps, nfft, discard, x_first=, out_first=, n_out=)` defaults to the CUDA
+    kernel."""
+    from . import _plan, fourier
+    if isinstance(h, torch.Tensor):
+        h = h.detach().cpu().numpy()
+    h = np.asarray(h)
+    if h.ndim != 1 or h.size == 0:
+        raise ValueError('oaconvolve_time_sharded: h must be 1-D with non-zero length')
+    world, rank = _world(group)
+    sh = oaconvolve_shard(n_samples, h.size, mode, world, rank)
+    if x_halo.ndim != 1 or x_halo.shape[0] != sh.sample1 - sh.sample0:
+        raise ValueError(f'rank {rank} expects a 1-D shard of {sh.sample1 - sh.sample0} samples, got {tuple(x_halo.shape)}')
+    nfft, discard = _plan.oaconvolve_plan(h.size)
+    hspec = _plan.oaconvolve_spectrum(h[None], nfft)
+    first, _ = _plan.oaconvolve_window(mode, n_samples, h.size)
+    kw = dict(x_first=sh.sample0, out_first=first + sh.out0, n_out=sh.out1 - sh.out0)
+    if compute is None:
+        from . import _arrays
+        xd, _ = _arrays.to_device(x_halo)
+        if xd.dtype != torch.complex64:
+            raise NotImplementedError(f'oaconvolve: only a complex64 signal is built (got {xd.dtype})')
+        y = fourier._oaconvolve_device(xd.reshape(1, -1), hspec, h.size, nfft, discard, **kw)[0]
+    else:
+        y = torch.as_tensor(compute(x_halo, hspec, h.size, nfft, discard, **kw))
+    if not gather or world == 1:
+        return y
+    sizes = [(lambda s: s.out1 - s.out0)(oaconvolve_shard(n_samples, h.size, mode, world, r)) for r in range(world)]
     return gather_rows(y, sizes, 0, group)

@@ -26,7 +26,7 @@ from . import _arrays, _lib, _plan
 from .util import Domain, get_input_domain
 from ._plan import INF
 
-__all__ = ['GraphedCall', 'fft', 'ifft', 'zero_stft_by_freq', 'stft', 'istft', 'ola_filter', 'oaresample', 'upfirdn', 'iq_to_stft_spectrogram', 'channelize_power', 'spectrogram', 'power_spectral_density', 'persistence_spectrum',
+__all__ = ['GraphedCall', 'fft', 'ifft', 'zero_stft_by_freq', 'stft', 'istft', 'ola_filter', 'oaresample', 'upfirdn', 'oaconvolve', 'iq_to_stft_spectrogram', 'channelize_power', 'spectrogram', 'power_spectral_density', 'persistence_spectrum',
            'fftfreq', 'get_window', 'equivalent_noise_bandwidth']
 
 fftfreq = _plan.fftfreq
@@ -591,6 +591,137 @@ def upfirdn(h, x, up=1, down=1, axis=-1, mode='constant', cval=0):
     x2, lead, trail = _arrays.as_channels(xd, axis)
     n_out = _plan.upfirdn_output_len(n_taps, x2.shape[1], up, down)
     y = _upfirdn_device(x2, table, n_taps, up, down, n_out=n_out)
+    return res.give_back(_arrays.restore_layout(y, lead, trail, 1))
+
+
+def _as_operand(a):
+    """a torch tensor as it is (host or device); anything else as a numpy array (no copy of arrays)"""
+    if isinstance(a, torch.Tensor):
+        return a
+    if hasattr(a, '__dlpack__') and not isinstance(a, np.ndarray):
+        return torch.from_dlpack(a)
+    return np.asarray(a)
+
+
+def _conv_axes(axes, nd: int) -> list[int]:
+    """scipy.fft's normalisation of `axes` (ValueError for out-of-range, repeated or empty axes)"""
+    if axes is None:
+        return list(range(nd))
+    import operator
+    ax = [operator.index(axes)] if np.ndim(axes) == 0 else [operator.index(a) for a in axes]
+    if not ax:
+        raise ValueError('when provided, axes cannot be empty')
+    ax = [a + nd if a < 0 else a for a in ax]
+    if any(a < 0 or a >= nd for a in ax):
+        raise ValueError('axes exceeds dimensionality of input')
+    if len(set(ax)) != len(ax):
+        raise ValueError('all axes must be unique')
+    return ax
+
+
+def _oaconvolve_roles(s1: tuple, s2: tuple, mode: str, axes):
+    """scipy.signal.oaconvolve's argument checks (ValueError) for non-empty operands of shapes s1, s2, and
+    what is not built (NotImplementedError).  Returns (a, signal_is_in1, per_row): the one convolved axis,
+    which operand is the signal (the longer along a; in1 on a tie) and whether the filter has one row per
+    signal row (else one row for all)."""
+    if mode not in ('full', 'same', 'valid'):
+        raise ValueError("acceptable mode flags are 'valid', 'same', or 'full'")
+    nd = len(s1)
+    ax = _conv_axes(axes, nd)
+    conv = [a for a in ax if s1[a] != 1 and s2[a] != 1]
+    if not all(s1[a] == s2[a] or s1[a] == 1 or s2[a] == 1 for a in range(nd) if a not in conv):
+        raise ValueError(f'incompatible shapes for in1 and in2: {s1} and {s2}')
+    if mode == 'valid' and not (all(s1[a] >= s2[a] for a in conv) or all(s2[a] >= s1[a] for a in conv)):
+        raise ValueError("For 'valid' mode, one must be at least as large as the other in every dimension")
+    if len(conv) > 1:
+        raise NotImplementedError(f'oaconvolve: convolution along more than one axis ({conv}) is not built')
+    # no axis with both sizes > 1: an elementwise product, i.e. a 1-tap convolution along the longest axis
+    a = conv[0] if conv else max(ax, key=lambda i: (max(s1[i], s2[i]), i))
+    signal_is_in1 = s1[a] >= s2[a]
+    xs, hs = (s1, s2) if signal_is_in1 else (s2, s1)
+    others = [i for i in range(nd) if i != a]
+    per_row = any(hs[i] != 1 for i in others)
+    if per_row and any(hs[i] != xs[i] for i in others):
+        raise NotImplementedError(f'oaconvolve: a filter of shape {hs} against a signal of shape {xs} (several filters '
+                                  f'per signal row, or a broadcast signal) is not built; the filter must have size 1 '
+                                  f'or the signal\'s size on every axis but {a}')
+    if hs[a] > _plan.OACONVOLVE_MAX_TAPS:
+        raise NotImplementedError(f'oaconvolve: both operands are longer than {_plan.OACONVOLVE_MAX_TAPS} samples '
+                                  f'along axis {a} ({s1[a]} and {s2[a]}); filters of more taps are not built')
+    return a, signal_is_in1, per_row
+
+
+def _oaconvolve_device(x2: torch.Tensor, hspec: np.ndarray, n_taps: int, nfft: int, discard: int, *,
+                       x_first: int = 0, out_first: int, n_out: int) -> torch.Tensor:
+    """(C, N) complex64 device rows holding global samples [x_first, x_first + N) -> (C, n_out) outputs
+    [out_first, out_first + n_out) of the full convolution.  `hspec`: (1 | C, nfft) complex64 spectrum rows
+    (_plan.oaconvolve_spectrum).  The kernel reads unit-stride rows: any other layout is copied first."""
+    C, N = x2.shape
+    if x2.stride(1) != 1 or (C > 1 and x2.stride(0) < N):
+        x2 = x2.contiguous()
+    y = torch.empty((C, n_out), dtype=torch.complex64, device=x2.device)
+    if n_out == 0 or C == 0:
+        return y
+    hd = torch.from_numpy(hspec).to(x2.device)
+    _lib.check(_lib.lib.iqw_oaconvolve_c64(
+        ctypes.c_void_p(x2.data_ptr()), C, N, x2.stride(0) if C > 1 else N, x_first, ctypes.c_void_p(hd.data_ptr()),
+        nfft if hspec.shape[0] > 1 else 0, n_taps, nfft, discard, out_first, n_out, ctypes.c_void_p(y.data_ptr()),
+        n_out, _stream_ptr(x2.device)))
+    return y
+
+
+def oaconvolve(in1, in2, mode='full', axes=None):
+    """convolve `in1` with `in2` along one axis by FFT overlap-save; the arguments, output shapes and
+    ValueErrors of scipy.signal.oaconvolve, which the reference forwards host arrays to
+    (fourier.py:1496-1509).  Along the convolved axis the longer operand is the signal (in1 on a tie) and
+    the other the filter, of M taps; the result comes back as the signal's kind (numpy, CPU or CUDA torch).
+
+    Built: a complex64 signal; a filter of any numeric dtype, real or complex, on the host or the device,
+    of at most 4097 taps; one convolved axis, with a filter of size 1 on every other axis (one filter for
+    every row) or of the signal's size there (one filter per row).  Anything else raises
+    NotImplementedError.  An empty operand gives an empty array of shape (0,).
+
+    Differences from scipy: the filter's spectrum fft(h, nfft) / nfft is computed in float64 and rounded
+    once to complex64, the device arithmetic is float32 and the result is always complex64 (scipy returns
+    complex128 for float64 operands).  The error follows the energy of each FFT block rather than each
+    output: |y - y_exact| stays within a small multiple of 2^-24 * log2(nfft) * max_k |fft(h, nfft)_k| *
+    rms(x over the block's nfft input samples) (DESIGN.md section 7).
+
+    Cost outside the kernel: every call computes the spectrum on the host (a filter on the device is copied
+    to the host first) and copies it to the device synchronously, rows x nfft x 8 bytes (64 KB per row at
+    nfft 8192).  Next to a long capture this is small; for many short calls with the same filter it is a
+    host round trip per call."""
+    in1, in2 = _as_operand(in1), _as_operand(in2)
+    s1, s2 = tuple(in1.shape), tuple(in2.shape)
+    if len(s1) != len(s2):
+        raise ValueError('in1 and in2 should have the same dimensionality')
+    if not s1:
+        raise NotImplementedError('oaconvolve: 0-d operands are not built')
+    if 0 in s1 or 0 in s2:
+        if isinstance(in1, torch.Tensor):
+            return torch.empty((0,), dtype=torch.complex64, device=in1.device)
+        return np.empty((0,), np.complex64)
+    a, signal_is_in1, per_row = _oaconvolve_roles(s1, s2, mode, axes)
+    x, h = (in1, in2) if signal_is_in1 else (in2, in1)
+    if x.dtype not in (np.complex64, torch.complex64):
+        raise NotImplementedError(f'oaconvolve: only a complex64 signal is built (got {x.dtype})')
+    if isinstance(h, torch.Tensor):
+        h = h.detach().cpu().numpy()
+    if not (np.issubdtype(h.dtype, np.number) or h.dtype == np.bool_):
+        raise NotImplementedError(f'oaconvolve: a filter of dtype {h.dtype} is not built')
+    n_taps = h.shape[a]
+    first, n_out = _plan.oaconvolve_window(mode, s1[a], s2[a])
+    nfft, discard = _plan.oaconvolve_plan(n_taps)
+    hspec = _plan.oaconvolve_spectrum(np.moveaxis(h, a, -1).reshape(-1, n_taps), nfft)
+    xd, res = _arrays.to_device(x)
+    if mode == 'same' and not signal_is_in1:
+        # scipy centres 'same' on in1's shape on every axis: where the (broadcast) filter in1 has size 1, the
+        # one row kept is the middle one of the signal
+        for i in range(xd.ndim):
+            if i != a and s1[i] != xd.shape[i]:
+                xd = xd.narrow(i, (xd.shape[i] - 1) // 2, 1)
+    x2, lead, trail = _arrays.as_channels(xd, a)
+    y = _oaconvolve_device(x2, hspec, n_taps, nfft, discard, out_first=first, n_out=n_out)
     return res.give_back(_arrays.restore_layout(y, lead, trail, 1))
 
 
