@@ -1,8 +1,9 @@
-// iqw_abi.cu -- version / error plumbing of the C-ABI (include/iqw_b200.h).
+// iqw_abi.cu -- version / error plumbing of the C-ABI (include/iqw_b200.h) and the per-device caches.
 #include <mutex>
 #include <vector>
 #include <string>
 #include <map>
+#include <tuple>
 #include <atomic>
 #include <cstring>
 #include "iqw_common.cuh"
@@ -25,6 +26,28 @@ int device_sm_count(int* sms) {
     IQW_CUDA_OK(cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev));
     if (dev < 64) cache[dev] = n;
     *sms = n;
+    return IQW_OK;
+}
+
+static std::mutex g_table_mutex;
+static std::map<std::tuple<int, int, int>, float2*> g_tables;   // (device, kind, param) -> table
+
+int device_table(TableKind kind, int param, size_t count, void (*init)(float2*, int, cudaStream_t), cudaStream_t stream,
+                 const float2** out) {
+    int dev = 0;
+    IQW_CUDA_OK(cudaGetDevice(&dev));
+    std::lock_guard<std::mutex> lock(g_table_mutex);
+    const auto key = std::make_tuple(dev, (int)kind, param);
+    auto it = g_tables.find(key);
+    if (it == g_tables.end()) {
+        float2* d = nullptr;
+        IQW_CUDA_OK(cudaMalloc(&d, sizeof(float2) * count));
+        init(d, param, stream);
+        IQW_CUDA_OK(cudaGetLastError());
+        IQW_CUDA_OK(cudaStreamSynchronize(stream));
+        it = g_tables.emplace(key, d).first;
+    }
+    *out = it->second;
     return IQW_OK;
 }
 

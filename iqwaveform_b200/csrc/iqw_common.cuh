@@ -1,9 +1,10 @@
-// iqw_common.cuh -- error plumbing and small device helpers shared by the three kernels.
+// iqw_common.cuh -- error and launch plumbing and small device helpers shared by the kernels.
 #pragma once
 #include <cuda_runtime.h>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdint>
+#include <type_traits>
 #include "../../include/iqw_b200.h"
 
 namespace iqw {
@@ -27,6 +28,43 @@ inline int fail(int code, const char* fmt, ...) {
     } while (0)
 
 int device_sm_count(int* sms);
+
+// log2(v) when v is a power of two, -1 otherwise (so a result < 1 rejects every v that is not a power of two >= 2)
+inline int log2_exact(long long v) {
+    if (v < 1 || (v & (v - 1))) return -1;
+    int l = 0;
+    while ((1ll << l) < v) ++l;
+    return l;
+}
+
+// Turns the runtime value v into a template argument: f(std::integral_constant<int, v>{}) when LO <= v <= HI,
+// fallback() otherwise.  Only the kernels that f names for LO..HI are instantiated.
+template <int LO, int HI, class F, class G>
+int dispatch(int v, F&& f, G&& fallback) {
+    if constexpr (LO > HI) return fallback();
+    else return v == LO ? f(std::integral_constant<int, LO>{}) : dispatch<LO + 1, HI>(v, f, fallback);
+}
+
+// Number of CTAs of `kern` that are resident at once (SMs x CTAs per SM) with `threads` threads and `smem` bytes of
+// dynamic shared memory, after raising the kernel's dynamic shared-memory limit to `smem`.
+template <class Kernel>
+int resident_ctas(Kernel kern, int threads, size_t smem, const char* name, long long* ctas) {
+    IQW_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int sms = 0, per_sm = 0;
+    if (int rc = device_sm_count(&sms)) return rc;
+    IQW_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem));
+    if (per_sm < 1)
+        return fail(IQW_ERR_CUDA, "%s (%d threads, %zu bytes of shared memory) does not fit on an SM", name, threads, smem);
+    *ctas = (long long)sms * per_sm;
+    return IQW_OK;
+}
+
+// Immutable float2 tables on the current device, built on first use: `init` launches the kernel that fills the
+// `count` entries of the table (kind, param) on `stream`; the stream is synchronised once, so that the table is
+// visible to every later stream.  `init` must not call device_table.
+enum TableKind { kFftTwiddles, kTwoPassTwiddles, kThreePassTwiddles, kStepTwiddles, kPfbRotation };
+int device_table(TableKind kind, int param, size_t count, void (*init)(float2* table, int param, cudaStream_t stream),
+                 cudaStream_t stream, const float2** out);
 
 // Every compute entry point launches on the device that OWNS its buffers, whatever device is current
 // in the calling thread (a tensor on cuda:1 while cuda:0 is current would otherwise be launched on the

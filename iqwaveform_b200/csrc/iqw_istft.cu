@@ -280,13 +280,10 @@ static int launch_ola_r(OlaArgs a, cudaStream_t stream) {
     } else {
         using C = StftCfg<LOG2N>;
         auto kern = ola_kernel<LOG2N, LOG2R>;
-        IQW_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-        int sms = 0, per_sm = 0;
-        if (int rc = device_sm_count(&sms)) return rc;
-        IQW_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, C::THREADS, C::SMEM));
-        if (per_sm < 1) return fail(IQW_ERR_CUDA, "ola kernel nfft=%d does not fit on an SM", C::N);
+        long long ctas = 0;
+        if (int rc = resident_ctas(kern, C::THREADS, C::SMEM, "ola kernel", &ctas)) return rc;
         constexpr int R = 1 << LOG2R;
-        long long streams = (long long)sms * per_sm * C::FPC;
+        long long streams = ctas * C::FPC;
         long long per_ch = streams / a.n_channels > 0 ? streams / a.n_channels : 1;
         const long long most = (a.n_frames + 16 * R - 1) / (16 * R);
         if (per_ch > most) per_ch = most;
@@ -299,31 +296,16 @@ static int launch_ola_r(OlaArgs a, cudaStream_t stream) {
     }
 }
 
-template <int LOG2N>
-static int launch_ola(const OlaArgs& a, int log2r, cudaStream_t s) {
-    switch (log2r) {
-        case 0: return launch_ola_r<LOG2N, 0>(a, s);
-        case 1: return launch_ola_r<LOG2N, 1>(a, s);
-        case 2: return launch_ola_r<LOG2N, 2>(a, s);
-        case 3: return launch_ola_r<LOG2N, 3>(a, s);
-        case 4: return launch_ola_r<LOG2N, 4>(a, s);
-    }
-    return fail(IQW_ERR_UNSUPPORTED, "ola: nfft/hop = %d: only 1, 2, 4, 8, 16 are built", 1 << log2r);
-}
-
 template <int LOG2N, int LOG2R, bool MASK, bool GAIN>
 static int launch_istft_r(IstftArgs a, cudaStream_t stream) {
     using C = StftCfg<LOG2N>;
     auto kern = istft_kernel<LOG2N, LOG2R, MASK, GAIN>;
-    IQW_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-    int sms = 0, per_sm = 0;
-    if (int rc = device_sm_count(&sms)) return rc;
-    IQW_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, C::THREADS, C::SMEM));
-    if (per_sm < 1) return fail(IQW_ERR_CUDA, "istft kernel nfft=%d does not fit on an SM", C::N);
+    long long ctas = 0;
+    if (int rc = resident_ctas(kern, C::THREADS, C::SMEM, "istft kernel", &ctas)) return rc;
     constexpr int R = 1 << LOG2R;
     // one frame range ("stream") per slot of the resident grid, but ranges of at least 16*R frames
     // so that the R-1 warm-up frames of a range stay a few per cent
-    long long streams = (long long)sms * per_sm * C::FPC;
+    long long streams = ctas * C::FPC;
     long long per_ch = streams / a.n_channels > 0 ? streams / a.n_channels : 1;
     const long long most = (a.n_frames + 16 * R - 1) / (16 * R);
     if (per_ch > most) per_ch = most;
@@ -348,18 +330,6 @@ static int launch_istft_m(const IstftArgs& a, cudaStream_t s) {
     }
 }
 
-template <int LOG2N>
-static int launch_istft(const IstftArgs& a, int log2r, cudaStream_t s) {
-    switch (log2r) {
-        case 0: return launch_istft_m<LOG2N, 0>(a, s);
-        case 1: return launch_istft_m<LOG2N, 1>(a, s);
-        case 2: return launch_istft_m<LOG2N, 2>(a, s);
-        case 3: return launch_istft_m<LOG2N, 3>(a, s);
-        case 4: return launch_istft_m<LOG2N, 4>(a, s);
-    }
-    return fail(IQW_ERR_UNSUPPORTED, "istft: nfft/hop = %d: only 1, 2, 4, 8, 16 are built", 1 << log2r);
-}
-
 }  // namespace iqw
 
 using namespace iqw;
@@ -369,16 +339,12 @@ static int istft_entry(const void* d_y, int64_t n_channels, int64_t n_frames, in
                        const void* d_bin_gain, float scale, int natural, void* d_out,
                        int64_t out_channel_stride, void* stream) {
     if (!d_y || !d_out) return fail(IQW_ERR_INVALID, "null pointer argument");
-    if (nfft < 2 || (nfft & (nfft - 1)))
-        return fail(IQW_ERR_UNSUPPORTED, "nfft=%d: only powers of two are built", nfft);
-    int log2n = 0;
-    while ((1 << log2n) < nfft) ++log2n;
+    const int log2n = log2_exact(nfft);
+    if (log2n < 1) return fail(IQW_ERR_UNSUPPORTED, "nfft=%d: only powers of two are built", nfft);
     if (log2n < 4 || log2n > 13)
         return fail(IQW_ERR_UNSUPPORTED, "istft: nfft=%d outside the built range 16..8192", nfft);
-    if (hop < 1 || hop > nfft || nfft % hop || ((nfft / hop) & (nfft / hop - 1)))
-        return fail(IQW_ERR_UNSUPPORTED, "istft: hop=%lld: nfft/hop must be 1, 2, 4, 8 or 16", (long long)hop);
-    int log2r = 0;
-    while (((int64_t)1 << log2r) < nfft / hop) ++log2r;
+    const int log2r = hop >= 1 && hop <= nfft && nfft % hop == 0 ? log2_exact(nfft / hop) : -1;
+    if (log2r < 0) return fail(IQW_ERR_UNSUPPORTED, "istft: hop=%lld: nfft/hop must be 1, 2, 4, 8 or 16", (long long)hop);
     if (n_channels < 1 || n_frames < 1) return fail(IQW_ERR_INVALID, "istft: need at least one channel and one frame");
     if (bin_lo < 0 || bin_hi > nfft || bin_lo > bin_hi) return fail(IQW_ERR_INVALID, "istft: bad bin range");
     if (y_bins != nfft && y_bins != bin_hi - bin_lo)
@@ -395,19 +361,14 @@ static int istft_entry(const void* d_y, int64_t n_channels, int64_t n_frames, in
     a.out = (float2*)d_out; a.out_ch_stride = out_channel_stride;
     a.streams_per_ch = a.frames_per_stream = 0;
     if (int rc = get_twiddles(log2n, s, &a.twiddle)) return rc;
-    switch (log2n) {
-        case 4: return launch_istft<4>(a, log2r, s);
-        case 5: return launch_istft<5>(a, log2r, s);
-        case 6: return launch_istft<6>(a, log2r, s);
-        case 7: return launch_istft<7>(a, log2r, s);
-        case 8: return launch_istft<8>(a, log2r, s);
-        case 9: return launch_istft<9>(a, log2r, s);
-        case 10: return launch_istft<10>(a, log2r, s);
-        case 11: return launch_istft<11>(a, log2r, s);
-        case 12: return launch_istft<12>(a, log2r, s);
-        case 13: return launch_istft<13>(a, log2r, s);
-    }
-    return fail(IQW_ERR_UNSUPPORTED, "istft: nfft=%d", nfft);
+    return dispatch<4, 13>(
+        log2n,
+        [&](auto L) {
+            return dispatch<0, 4>(log2r, [&](auto R) { return launch_istft_m<L, R>(a, s); }, [&] {
+                return fail(IQW_ERR_UNSUPPORTED, "istft: nfft/hop = %d: only 1, 2, 4, 8, 16 are built", 1 << log2r);
+            });
+        },
+        [&] { return fail(IQW_ERR_UNSUPPORTED, "istft: nfft=%d", nfft); });
 }
 
 extern "C" int iqw_istft_c64(const void* d_y, int64_t n_channels, int64_t n_frames, int64_t y_channel_stride,
@@ -434,16 +395,13 @@ extern "C" int iqw_ola_filter_c64(const void* d_x, int64_t n_channels, int64_t n
                                   void* stream) {
     iqw::DeviceGuard _dev_guard(d_x);
     if (!d_x || !d_out || !d_window) return fail(IQW_ERR_INVALID, "null pointer argument");
-    if (nfft < 2 || (nfft & (nfft - 1)))
-        return fail(IQW_ERR_UNSUPPORTED, "nfft=%d: only powers of two are built", nfft);
-    int log2n = 0;
-    while ((1 << log2n) < nfft) ++log2n;
+    const int log2n = log2_exact(nfft);
+    if (log2n < 1) return fail(IQW_ERR_UNSUPPORTED, "nfft=%d: only powers of two are built", nfft);
     if (log2n < 4 || log2n > 13)
         return fail(IQW_ERR_UNSUPPORTED, "ola_filter: nfft=%d outside the built range 16..8192", nfft);
-    if (hop < 1 || hop > nfft || nfft % hop || ((nfft / hop) & (nfft / hop - 1)))
+    const int log2r = hop >= 1 && hop <= nfft && nfft % hop == 0 ? log2_exact(nfft / hop) : -1;
+    if (log2r < 0)
         return fail(IQW_ERR_UNSUPPORTED, "ola_filter: hop=%lld: nfft/hop must be 1, 2, 4, 8 or 16", (long long)hop);
-    int log2r = 0;
-    while (((int64_t)1 << log2r) < nfft / hop) ++log2r;
     if (n_channels < 1 || n_frames < 1) return fail(IQW_ERR_INVALID, "ola_filter: need at least one channel and one frame");
     if ((n_frames - 1) * hop + nfft > n_samples) return fail(IQW_ERR_INVALID, "ola_filter: frames run past the samples");
     if (bin_lo < 0 || bin_hi > nfft || bin_lo > bin_hi) return fail(IQW_ERR_INVALID, "ola_filter: bad bin range");
@@ -456,17 +414,12 @@ extern "C" int iqw_ola_filter_c64(const void* d_x, int64_t n_channels, int64_t n
     a.out = (float2*)d_out; a.out_ch_stride = out_channel_stride;
     a.streams_per_ch = a.frames_per_stream = 0;
     if (int rc = get_twiddles(log2n, s, &a.twiddle)) return rc;
-    switch (log2n) {
-        case 4: return launch_ola<4>(a, log2r, s);
-        case 5: return launch_ola<5>(a, log2r, s);
-        case 6: return launch_ola<6>(a, log2r, s);
-        case 7: return launch_ola<7>(a, log2r, s);
-        case 8: return launch_ola<8>(a, log2r, s);
-        case 9: return launch_ola<9>(a, log2r, s);
-        case 10: return launch_ola<10>(a, log2r, s);
-        case 11: return launch_ola<11>(a, log2r, s);
-        case 12: return launch_ola<12>(a, log2r, s);
-        case 13: return launch_ola<13>(a, log2r, s);
-    }
-    return fail(IQW_ERR_UNSUPPORTED, "ola_filter: nfft=%d", nfft);
+    return dispatch<4, 13>(
+        log2n,
+        [&](auto L) {
+            return dispatch<0, 4>(log2r, [&](auto R) { return launch_ola_r<L, R>(a, s); }, [&] {
+                return fail(IQW_ERR_UNSUPPORTED, "ola: nfft/hop = %d: only 1, 2, 4, 8, 16 are built", 1 << log2r);
+            });
+        },
+        [&] { return fail(IQW_ERR_UNSUPPORTED, "ola_filter: nfft=%d", nfft); });
 }

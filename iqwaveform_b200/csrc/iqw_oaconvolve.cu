@@ -153,14 +153,11 @@ static int launch_oaconvolve_r(OaconvArgs a, cudaStream_t stream) {
     } else {
         using C = StftCfg<LOG2N>;
         auto kern = oaconvolve_kernel<LOG2N, LOG2R>;
-        IQW_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-        int sms = 0, per_sm = 0;
-        if (int rc = device_sm_count(&sms)) return rc;
-        IQW_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, C::THREADS, C::SMEM));
-        if (per_sm < 1) return fail(IQW_ERR_CUDA, "oaconvolve kernel nfft=%d does not fit on an SM", C::N);
+        long long ctas = 0;
+        if (int rc = resident_ctas(kern, C::THREADS, C::SMEM, "oaconvolve kernel", &ctas)) return rc;
         // one block range per slot of the resident grid, of at least 4 blocks so that the first,
         // unhidden load of a range stays a small part of it
-        const long long streams = (long long)sms * per_sm * C::FPC;
+        const long long streams = ctas * C::FPC;
         long long per_ch = streams / a.n_channels > 0 ? streams / a.n_channels : 1;
         const long long most = (a.n_blocks + 3) / 4;
         if (per_ch > most) per_ch = most;
@@ -174,17 +171,6 @@ static int launch_oaconvolve_r(OaconvArgs a, cudaStream_t stream) {
     }
 }
 
-template <int LOG2N>
-static int launch_oaconvolve(const OaconvArgs& a, int log2r, cudaStream_t s) {
-    switch (log2r) {
-        case 1: return launch_oaconvolve_r<LOG2N, 1>(a, s);
-        case 2: return launch_oaconvolve_r<LOG2N, 2>(a, s);
-        case 3: return launch_oaconvolve_r<LOG2N, 3>(a, s);
-        case 4: return launch_oaconvolve_r<LOG2N, 4>(a, s);
-    }
-    return fail(IQW_ERR_UNSUPPORTED, "oaconvolve: nfft/discard = %d: only 2, 4, 8, 16 are built", 1 << log2r);
-}
-
 }  // namespace iqw
 
 extern "C" int iqw_oaconvolve_c64(const void* d_x, int64_t n_channels, int64_t n_in, int64_t x_channel_stride,
@@ -192,17 +178,12 @@ extern "C" int iqw_oaconvolve_c64(const void* d_x, int64_t n_channels, int64_t n
                                   int32_t n_taps, int32_t nfft, int32_t discard, int64_t out_first, int64_t n_out,
                                   void* d_out, int64_t out_channel_stride, void* stream) {
     using namespace iqw;
-    if (nfft < 2 || (nfft & (nfft - 1)))
-        return fail(IQW_ERR_UNSUPPORTED, "oaconvolve: nfft=%d: only powers of two are built", nfft);
-    int log2n = 0;
-    while ((1 << log2n) < nfft) ++log2n;
+    const int log2n = log2_exact(nfft);
+    if (log2n < 1) return fail(IQW_ERR_UNSUPPORTED, "oaconvolve: nfft=%d: only powers of two are built", nfft);
     if (log2n < 4 || log2n > 13)
         return fail(IQW_ERR_UNSUPPORTED, "oaconvolve: nfft=%d outside the built range 16..8192", nfft);
-    if (discard < 1 || discard >= nfft || nfft % discard || ((nfft / discard) & (nfft / discard - 1)))
-        return fail(IQW_ERR_UNSUPPORTED, "oaconvolve: discard=%d: nfft/discard must be 2, 4, 8 or 16", discard);
-    int log2r = 0;
-    while ((1 << log2r) < nfft / discard) ++log2r;
-    if (log2r > 4)
+    const int log2r = discard >= 1 && discard < nfft && nfft % discard == 0 ? log2_exact(nfft / discard) : -1;
+    if (log2r < 0 || log2r > 4)
         return fail(IQW_ERR_UNSUPPORTED, "oaconvolve: discard=%d: nfft/discard must be 2, 4, 8 or 16", discard);
     if (n_taps < 1 || discard < n_taps - 1)
         return fail(IQW_ERR_INVALID, "oaconvolve: need 1 <= n_taps <= discard + 1 (n_taps %d, discard %d)", n_taps,
@@ -233,17 +214,12 @@ extern "C" int iqw_oaconvolve_c64(const void* d_x, int64_t n_channels, int64_t n
     a.n_blocks = (out_first + n_out - 1) / hop - a.b_first + 1;
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     if (int rc = get_twiddles(log2n, s, &a.twiddle)) return rc;
-    switch (log2n) {
-        case 4: return launch_oaconvolve<4>(a, log2r, s);
-        case 5: return launch_oaconvolve<5>(a, log2r, s);
-        case 6: return launch_oaconvolve<6>(a, log2r, s);
-        case 7: return launch_oaconvolve<7>(a, log2r, s);
-        case 8: return launch_oaconvolve<8>(a, log2r, s);
-        case 9: return launch_oaconvolve<9>(a, log2r, s);
-        case 10: return launch_oaconvolve<10>(a, log2r, s);
-        case 11: return launch_oaconvolve<11>(a, log2r, s);
-        case 12: return launch_oaconvolve<12>(a, log2r, s);
-        case 13: return launch_oaconvolve<13>(a, log2r, s);
-    }
-    return fail(IQW_ERR_UNSUPPORTED, "oaconvolve: nfft=%d", nfft);
+    return dispatch<4, 13>(
+        log2n,
+        [&](auto L) {
+            return dispatch<1, 4>(log2r, [&](auto R) { return launch_oaconvolve_r<L, R>(a, s); }, [&] {
+                return fail(IQW_ERR_UNSUPPORTED, "oaconvolve: nfft/discard = %d: only 2, 4, 8, 16 are built", 1 << log2r);
+            });
+        },
+        [&] { return fail(IQW_ERR_UNSUPPORTED, "oaconvolve: nfft=%d", nfft); });
 }

@@ -22,9 +22,6 @@
 //
 // Determinism: a frame's arithmetic depends only on its L samples, the taps and its global index m, never on
 // where a call starts (frame_first), so time shards concatenate to the bits of one call.
-#include <map>
-#include <mutex>
-#include <utility>
 #include "iqw_stft.cuh"
 
 namespace iqw {
@@ -139,39 +136,14 @@ __global__ void pfb_rot_init_kernel(float2* rot, int n) {
     }
 }
 
-static std::mutex g_rot_mutex;
-static std::map<std::pair<int, int>, float2*> g_rot_cache;
-
-static int get_rotation(int log2n, cudaStream_t stream, const float2** out) {
-    int dev = 0;
-    IQW_CUDA_OK(cudaGetDevice(&dev));
-    std::lock_guard<std::mutex> lock(g_rot_mutex);
-    auto key = std::make_pair(dev, log2n);
-    auto it = g_rot_cache.find(key);
-    if (it == g_rot_cache.end()) {
-        float2* d = nullptr;
-        IQW_CUDA_OK(cudaMalloc(&d, sizeof(float2) << log2n));
-        pfb_rot_init_kernel<<<8, 256, 0, stream>>>(d, 1 << log2n);
-        IQW_CUDA_OK(cudaGetLastError());
-        IQW_CUDA_OK(cudaStreamSynchronize(stream));   // one-time: visible to every later stream
-        it = g_rot_cache.emplace(key, d).first;
-    }
-    *out = it->second;
-    return IQW_OK;
-}
-
 template <int LOG2N>
 static int launch_pfb(PfbArgs a, cudaStream_t stream) {
     using C = StftCfg<LOG2N>;
     auto kern = pfb_kernel<LOG2N>;
-    IQW_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-    int sms = 0, per_sm = 0;
-    if (int rc = device_sm_count(&sms)) return rc;
-    IQW_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, C::THREADS, C::SMEM));
-    if (per_sm < 1) return fail(IQW_ERR_CUDA, "pfb kernel K=%d does not fit on an SM", C::N);
+    long long grid = 0;
+    if (int rc = resident_ctas(kern, C::THREADS, C::SMEM, "pfb kernel", &grid)) return rc;
     a.groups_per_ch = (a.n_frames + C::FPC - 1) / C::FPC;
     a.n_groups = a.groups_per_ch * a.n_channels;
-    long long grid = (long long)sms * per_sm;
     if (grid > a.n_groups) grid = a.n_groups;
     { IQW_PROFILE("pfb_kernel", stream); kern<<<(unsigned)grid, C::THREADS, C::SMEM, stream>>>(a); }
     IQW_CUDA_OK(cudaGetLastError());
@@ -185,10 +157,8 @@ extern "C" int iqw_pfb_channelize_c64(const void* d_x, int64_t n_channels, int64
                                       int64_t frame_first, int64_t n_frames, void* d_out, int64_t out_channel_stride,
                                       void* stream) {
     using namespace iqw;
-    if (nfft < 2 || (nfft & (nfft - 1)))
-        return fail(IQW_ERR_UNSUPPORTED, "pfb_channelize: nfft=%d: only powers of two are built", nfft);
-    int log2n = 0;
-    while ((1 << log2n) < nfft) ++log2n;
+    const int log2n = log2_exact(nfft);
+    if (log2n < 1) return fail(IQW_ERR_UNSUPPORTED, "pfb_channelize: nfft=%d: only powers of two are built", nfft);
     if (log2n < 4 || log2n > 13)
         return fail(IQW_ERR_UNSUPPORTED, "pfb_channelize: nfft=%d outside the built range 16..8192", nfft);
     if (n_taps < 1) return fail(IQW_ERR_INVALID, "pfb_channelize: n_taps=%d: need at least one tap", n_taps);
@@ -225,18 +195,10 @@ extern "C" int iqw_pfb_channelize_c64(const void* d_x, int64_t n_channels, int64
     a.n_channels = (int)n_channels;
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     if (int rc = get_twiddles(log2n, s, &a.twiddle)) return rc;
-    if (int rc = get_rotation(log2n, s, &a.rot)) return rc;
-    switch (log2n) {
-        case 4: return launch_pfb<4>(a, s);
-        case 5: return launch_pfb<5>(a, s);
-        case 6: return launch_pfb<6>(a, s);
-        case 7: return launch_pfb<7>(a, s);
-        case 8: return launch_pfb<8>(a, s);
-        case 9: return launch_pfb<9>(a, s);
-        case 10: return launch_pfb<10>(a, s);
-        case 11: return launch_pfb<11>(a, s);
-        case 12: return launch_pfb<12>(a, s);
-        case 13: return launch_pfb<13>(a, s);
-    }
-    return fail(IQW_ERR_UNSUPPORTED, "pfb_channelize: nfft=%d", nfft);
+    if (int rc = device_table(kPfbRotation, log2n, (size_t)1 << log2n,
+                              [](float2* d, int log2n, cudaStream_t s) { pfb_rot_init_kernel<<<8, 256, 0, s>>>(d, 1 << log2n); },
+                              s, &a.rot))
+        return rc;
+    return dispatch<4, 13>(log2n, [&](auto L) { return launch_pfb<L>(a, s); },
+                           [&] { return fail(IQW_ERR_UNSUPPORTED, "pfb_channelize: nfft=%d", nfft); });
 }

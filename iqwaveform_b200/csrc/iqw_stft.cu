@@ -14,9 +14,6 @@
 // re-read from L1/L2, never from HBM.  Between passes the values are exchanged through padded
 // ping-pong shared-memory buffers; the per-pass twiddle tables live in shared memory, laid out
 // [r][i] so that a warp reads consecutive entries.
-#include <mutex>
-#include <map>
-#include <utility>
 #include "iqw_stft.cuh"
 
 namespace iqw {
@@ -222,40 +219,20 @@ __global__ void twiddle_init_kernel(float2* tw, int log2n) {
     }
 }
 
-static std::mutex g_tw_mutex;
-static std::map<std::pair<int, int>, float2*> g_tw_cache;
-
 int get_twiddles(int log2n, cudaStream_t stream, const float2** out) {
-    int dev = 0;
-    IQW_CUDA_OK(cudaGetDevice(&dev));
-    std::lock_guard<std::mutex> lock(g_tw_mutex);
-    auto key = std::make_pair(dev, log2n);
-    auto it = g_tw_cache.find(key);
-    if (it == g_tw_cache.end()) {
-        float2* d = nullptr;
-        const int n = plan_tw_size(log2n) + 16;
-        IQW_CUDA_OK(cudaMalloc(&d, sizeof(float2) * n));
-        twiddle_init_kernel<<<8, 256, 0, stream>>>(d, log2n);
-        IQW_CUDA_OK(cudaGetLastError());
-        IQW_CUDA_OK(cudaStreamSynchronize(stream));   // one-time: visible to every later stream
-        it = g_tw_cache.emplace(key, d).first;
-    }
-    *out = it->second;
-    return IQW_OK;
+    return device_table(kFftTwiddles, log2n, plan_tw_size(log2n) + 16,
+                        [](float2* d, int log2n, cudaStream_t s) { twiddle_init_kernel<<<8, 256, 0, s>>>(d, log2n); },
+                        stream, out);
 }
 
 template <int LOG2N, int MODE, bool FULLBAND>
 static int launch_stft_band(StftArgs a, cudaStream_t stream) {
     using C = StftCfg<LOG2N>;
     auto kern = stft_kernel<LOG2N, MODE, FULLBAND>;
-    IQW_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-    int sms = 0, per_sm = 0;
-    if (int rc = device_sm_count(&sms)) return rc;
-    IQW_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, C::THREADS, C::SMEM));
-    if (per_sm < 1) return fail(IQW_ERR_CUDA, "stft kernel nfft=%d does not fit on an SM", C::N);
+    long long grid = 0;
+    if (int rc = resident_ctas(kern, C::THREADS, C::SMEM, "stft kernel", &grid)) return rc;
     a.groups_per_ch = (a.n_frames + C::FPC - 1) / C::FPC;
     a.n_groups = a.groups_per_ch * a.n_channels;
-    long long grid = (long long)sms * per_sm;
     if (grid > a.n_groups) grid = a.n_groups;
     { IQW_PROFILE("stft_kernel", stream); kern<<<(unsigned)grid, C::THREADS, C::SMEM, stream>>>(a); }
     IQW_CUDA_OK(cudaGetLastError());
@@ -269,28 +246,14 @@ static int launch_stft(const StftArgs& a, cudaStream_t stream) {
 }
 
 template <int LOG2N>
-static int launch_stft_mode(const StftArgs& a, int mode, cudaStream_t s) {
-    switch (mode) {
-        case IQW_STFT_COMPLEX: return launch_stft<LOG2N, IQW_STFT_COMPLEX>(a, s);
-        case IQW_STFT_POWER: return launch_stft<LOG2N, IQW_STFT_POWER>(a, s);
-        case IQW_STFT_DB: return launch_stft<LOG2N, IQW_STFT_DB>(a, s);
-    }
-    return fail(IQW_ERR_INVALID, "unknown stft mode %d", mode);
-}
-
-template <int LOG2N>
 static int launch_stft_reduce(StftArgs a, const ReducePlan& st, float* out, void* ws, size_t ws_bytes, cudaStream_t stream) {
     using C = StftCfg<LOG2N>;
     auto kern = stft_kernel<LOG2N, kStftReduce, true>;
-    IQW_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-    int sms = 0, per_sm = 0;
-    if (int rc = device_sm_count(&sms)) return rc;
-    IQW_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, C::THREADS, C::SMEM));
-    if (per_sm < 1) return fail(IQW_ERR_CUDA, "stft reduce kernel nfft=%d does not fit on an SM", C::N);
+    long long grid = 0;
+    if (int rc = resident_ctas(kern, C::THREADS, C::SMEM, "stft reduce kernel", &grid)) return rc;
     a.n_channels = 1;
     a.groups_per_ch = (a.n_frames + C::FPC - 1) / C::FPC;
     a.n_groups = a.groups_per_ch;
-    long long grid = (long long)sms * per_sm;
     if (grid > a.n_groups) grid = a.n_groups;
     const long long n_parts = grid * C::FPC;
     const size_t need = (size_t)n_parts * C::N * (2 * sizeof(float) + sizeof(double));
@@ -357,7 +320,8 @@ extern "C" int iqw_stft_reduce_c64(const void* d_x, int64_t n_channels, int64_t 
                                    float* d_out, void* d_workspace, size_t workspace_bytes, void* stream) {
     iqw::DeviceGuard _dev_guard(d_x);
     if (!d_x || !d_window || !d_out || !stats) return fail(IQW_ERR_INVALID, "null pointer argument");
-    if (nfft < 16 || nfft > 8192 || (nfft & (nfft - 1)))
+    const int log2n = log2_exact(nfft);
+    if (log2n < 4 || log2n > 13)
         return fail(IQW_ERR_UNSUPPORTED, "iqw_stft_reduce_c64: nfft=%d: powers of two from 16 to 8192 are built", nfft);
     if (hop < 1 || n_channels < 1 || n_frames < 1) return fail(IQW_ERR_INVALID, "need hop, n_channels, n_frames >= 1");
     if ((n_frames - 1) * hop + nfft > n_samples)
@@ -371,8 +335,6 @@ extern "C" int iqw_stft_reduce_c64(const void* d_x, int64_t n_channels, int64_t 
             return fail(IQW_ERR_UNSUPPORTED, "iqw_stft_reduce_c64 takes mean / max / min only (order statistics need the spectrogram)");
         st.kind[t] = stats[t].kind;
     }
-    int log2n = 0;
-    while ((1 << log2n) < nfft) ++log2n;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const int nb = bin_hi - bin_lo;
     for (int64_t c = 0; c < n_channels; ++c) {
@@ -393,28 +355,17 @@ extern "C" int iqw_stft_reduce_c64(const void* d_x, int64_t n_channels, int64_t 
         bool done = false;
         if (int rc2 = launch_stft_reduce_two_pass(a, log2n, st, out, d_workspace, workspace_bytes, s, &done)) return rc2;
         if (done) continue;
-        int rc = IQW_ERR_UNSUPPORTED;
-        switch (log2n) {
-            case 4: rc = launch_stft_reduce<4>(a, st, out, d_workspace, workspace_bytes, s); break;
-            case 5: rc = launch_stft_reduce<5>(a, st, out, d_workspace, workspace_bytes, s); break;
-            case 6: rc = launch_stft_reduce<6>(a, st, out, d_workspace, workspace_bytes, s); break;
-            case 7: rc = launch_stft_reduce<7>(a, st, out, d_workspace, workspace_bytes, s); break;
-            case 8: rc = launch_stft_reduce<8>(a, st, out, d_workspace, workspace_bytes, s); break;
-            case 9: rc = launch_stft_reduce<9>(a, st, out, d_workspace, workspace_bytes, s); break;
-            case 10: rc = launch_stft_reduce<10>(a, st, out, d_workspace, workspace_bytes, s); break;
-            case 11: rc = launch_stft_reduce<11>(a, st, out, d_workspace, workspace_bytes, s); break;
-            case 12: rc = launch_stft_reduce<12>(a, st, out, d_workspace, workspace_bytes, s); break;
-            case 13: rc = launch_stft_reduce<13>(a, st, out, d_workspace, workspace_bytes, s); break;
-        }
+        const int rc = dispatch<4, 13>(
+            log2n, [&](auto L) { return launch_stft_reduce<L>(a, st, out, d_workspace, workspace_bytes, s); },
+            [] { return IQW_ERR_UNSUPPORTED; });
         if (rc) return rc;
     }
     return IQW_OK;
 }
 
 extern "C" size_t iqw_stft_workspace_bytes(int32_t nfft, int64_t n_channels, int64_t n_frames) {
-    if (nfft < 2 || (nfft & (nfft - 1))) return 0;
-    int log2n = 0;
-    while ((1 << log2n) < nfft) ++log2n;
+    const int log2n = log2_exact(nfft);
+    if (log2n < 1) return 0;
     // the four-step path's scratch (also the fallback for unaligned captures) or the cluster kernels' exchange
     // scratch, whichever is larger
     const size_t four_step = stft_large_workspace_bytes(log2n, n_channels, n_frames);
@@ -429,10 +380,8 @@ extern "C" int iqw_stft_c64(const void* d_x, int64_t n_channels, int64_t n_sampl
                             size_t workspace_bytes, void* stream) {
     iqw::DeviceGuard _dev_guard(d_x);
     if (!d_x || !d_window || !d_out) return fail(IQW_ERR_INVALID, "null pointer argument");
-    if (nfft < 2 || (nfft & (nfft - 1)))
-        return fail(IQW_ERR_UNSUPPORTED, "nfft=%d: only powers of two are built", nfft);
-    int log2n = 0;
-    while ((1 << log2n) < nfft) ++log2n;
+    const int log2n = log2_exact(nfft);
+    if (log2n < 1) return fail(IQW_ERR_UNSUPPORTED, "nfft=%d: only powers of two are built", nfft);
     if (log2n < 4 || log2n > 16)
         return fail(IQW_ERR_UNSUPPORTED, "nfft=%d outside the built range 16..65536", nfft);
     if (hop < 1) return fail(IQW_ERR_INVALID, "hop=%lld must be >= 1", (long long)hop);
@@ -473,18 +422,7 @@ extern "C" int iqw_stft_c64(const void* d_x, int64_t n_channels, int64_t n_sampl
     if (log2n > 13) return launch_stft_large(a, log2n, mode, d_workspace, workspace_bytes, s);
     if (stft_two_pass_wanted(log2n)) return launch_stft_two_pass(a, log2n, mode, s);
     if (int rc = get_twiddles(log2n, s, &a.twiddle)) return rc;
-
-    switch (log2n) {
-        case 4: return launch_stft_mode<4>(a, mode, s);
-        case 5: return launch_stft_mode<5>(a, mode, s);
-        case 6: return launch_stft_mode<6>(a, mode, s);
-        case 7: return launch_stft_mode<7>(a, mode, s);
-        case 8: return launch_stft_mode<8>(a, mode, s);
-        case 9: return launch_stft_mode<9>(a, mode, s);
-        case 10: return launch_stft_mode<10>(a, mode, s);
-        case 11: return launch_stft_mode<11>(a, mode, s);
-        case 12: return launch_stft_mode<12>(a, mode, s);
-        case 13: return launch_stft_mode<13>(a, mode, s);
-    }
-    return fail(IQW_ERR_UNSUPPORTED, "nfft=%d", nfft);
+    return dispatch<4, 13>(
+        log2n, [&](auto L) { return dispatch_stft_mode(mode, [&](auto M) { return launch_stft<L, M>(a, s); }); },
+        [&] { return fail(IQW_ERR_UNSUPPORTED, "nfft=%d", nfft); });
 }

@@ -31,6 +31,12 @@ struct StftArgs {
 
 constexpr int kStftReduce = 3;   // internal mode of stft_kernel, next to IQW_STFT_COMPLEX / POWER / DB
 
+// f(std::integral_constant<int, mode>{}) for the output modes IQW_STFT_COMPLEX / POWER / DB
+template <class F>
+int dispatch_stft_mode(int mode, F&& f) {
+    return dispatch<IQW_STFT_COMPLEX, IQW_STFT_DB>(mode, f, [&] { return fail(IQW_ERR_INVALID, "unknown stft mode %d", mode); });
+}
+
 // geometry of the in-CTA FFT (shared by the forward kernel, iqw_stft.cu, and the inverse one,
 // iqw_istft.cu)
 template <int LOG2N>
@@ -87,7 +93,7 @@ bool stft_two_pass_wanted(int log2n);
 int launch_stft_two_pass(const StftArgs& a, int log2n, int mode, cudaStream_t stream);
 
 // reducible statistics fused into the two-pass kernel (warp-specialised; iqw_stft2p.cu).  flags: bit 0 max, bit 1 min,
-// bit 2 sum; IQW_ERR_UNSUPPORTED for all three at once.  Leaves *n_parts partial rows in a.part_max / min / sum.
+// bit 2 sum; IQW_ERR_UNSUPPORTED (no error message) outside nfft 1024..4096 and flags 1..7.  Leaves *n_parts partial rows in a.part_max / min / sum.
 int launch_stft_two_pass_reduce(const StftArgs& a, int log2n, int flags, long long* n_parts, cudaStream_t stream);
 
 // nfft 8192 .. 65536 in one pass: frame in (distributed) shared memory, cluster of 1 / 1 / 2 / 4 CTAs (iqw_stft3p.cu)

@@ -18,9 +18,6 @@
 // of frames, so the overlapped half of consecutive frames is re-read from L2 a few microseconds after its
 // first use.  Rows of M are padded by two elements (a row is an odd number of 16-byte units), which makes
 // both the 128-bit row stores and the 64-bit column loads conflict-free.
-#include <mutex>
-#include <map>
-#include <utility>
 #include <atomic>
 #include "iqw_stft.cuh"
 
@@ -264,27 +261,14 @@ __global__ void twiddle2p_init_kernel(float2* tw, int n, int ra, int rb) {
     }
 }
 
-static std::mutex g_tw2_mutex;
-static std::map<std::pair<int, int>, float2*> g_tw2_cache;
-
 template <int LOG2N>
 static int get_twiddles2p(cudaStream_t stream, const float2** out) {
-    using C = P2Cfg<LOG2N, true>;
-    int dev = 0;
-    IQW_CUDA_OK(cudaGetDevice(&dev));
-    std::lock_guard<std::mutex> lock(g_tw2_mutex);
-    auto key = std::make_pair(dev, LOG2N);
-    auto it = g_tw2_cache.find(key);
-    if (it == g_tw2_cache.end()) {
-        float2* d = nullptr;
-        IQW_CUDA_OK(cudaMalloc(&d, sizeof(float2) * C::TW));
-        twiddle2p_init_kernel<<<16, 256, 0, stream>>>(d, C::N, C::RA, C::RB);
-        IQW_CUDA_OK(cudaGetLastError());
-        IQW_CUDA_OK(cudaStreamSynchronize(stream));   // one-time: visible to every later stream
-        it = g_tw2_cache.emplace(key, d).first;
-    }
-    *out = it->second;
-    return IQW_OK;
+    return device_table(kTwoPassTwiddles, LOG2N, P2Cfg<LOG2N, true>::TW,
+                        [](float2* d, int, cudaStream_t s) {
+                            using C = P2Cfg<LOG2N, true>;
+                            twiddle2p_init_kernel<<<16, 256, 0, s>>>(d, C::N, C::RA, C::RB);
+                        },
+                        stream, out);
 }
 
 template <int LOG2N, int MODE, bool FULLBAND, bool STAGED>
@@ -292,13 +276,9 @@ static int launch2p_staged(StftArgs a, cudaStream_t stream) {
     using C = P2Cfg<LOG2N, STAGED>;
     auto kern = stft2p_kernel<LOG2N, MODE, FULLBAND, STAGED>;
     if (int rc = get_twiddles2p<LOG2N>(stream, &a.twiddle)) return rc;
-    IQW_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-    int sms = 0, per_sm = 0;
-    if (int rc = device_sm_count(&sms)) return rc;
-    IQW_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, C::THREADS, C::SMEM));
-    if (per_sm < 1) return fail(IQW_ERR_CUDA, "two-pass stft kernel nfft=%d does not fit on an SM", C::N);
+    long long grid = 0;
+    if (int rc = resident_ctas(kern, C::THREADS, C::SMEM, "two-pass stft kernel", &grid)) return rc;
     const long long total = (long long)a.n_channels * a.n_frames;
-    long long grid = (long long)sms * per_sm;
     const long long need = (total + C::SLOTS - 1) / C::SLOTS;
     if (grid > need) grid = need;
     { IQW_PROFILE("stft_kernel", stream); kern<<<(unsigned)grid, C::THREADS, C::SMEM, stream>>>(a); }
@@ -322,15 +302,9 @@ static int launch2p_band(const StftArgs& a, cudaStream_t stream) {
 template <int LOG2N>
 static int launch2p(const StftArgs& a, int mode, cudaStream_t s) {
     const bool full = a.bin_lo == 0 && a.bin_hi == (1 << LOG2N);
-    switch (mode) {
-        case IQW_STFT_COMPLEX:
-            return full ? launch2p_band<LOG2N, IQW_STFT_COMPLEX, true>(a, s) : launch2p_band<LOG2N, IQW_STFT_COMPLEX, false>(a, s);
-        case IQW_STFT_POWER:
-            return full ? launch2p_band<LOG2N, IQW_STFT_POWER, true>(a, s) : launch2p_band<LOG2N, IQW_STFT_POWER, false>(a, s);
-        case IQW_STFT_DB:
-            return full ? launch2p_band<LOG2N, IQW_STFT_DB, true>(a, s) : launch2p_band<LOG2N, IQW_STFT_DB, false>(a, s);
-    }
-    return fail(IQW_ERR_INVALID, "unknown stft mode %d", mode);
+    return dispatch_stft_mode(mode, [&](auto M) {
+        return full ? launch2p_band<LOG2N, M, true>(a, s) : launch2p_band<LOG2N, M, false>(a, s);
+    });
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -608,29 +582,13 @@ static int launch2p_reduce_flags(StftArgs a, long long* n_parts, cudaStream_t st
     return IQW_OK;
 }
 
-// flags: bit 0 max, bit 1 min, bit 2 sum; returns IQW_ERR_UNSUPPORTED when all three are wanted (the caller then
-// takes the three-pass kernel, whose 16 values per thread leave room for all of them)
+// flags: bit 0 max, bit 1 min, bit 2 sum; returns IQW_ERR_UNSUPPORTED, without an error message, for an nfft or
+// flags that are not built here (the caller then takes the three-pass kernel)
 int launch_stft_two_pass_reduce(const StftArgs& a, int log2n, int flags, long long* n_parts, cudaStream_t stream) {
-#define IQW_R2(L, F) return launch2p_reduce_flags<L, F>(a, n_parts, stream)
-#define IQW_R2F(L)                                    \
-    switch (flags) {                                  \
-        case 1: IQW_R2(L, 1);                         \
-        case 2: IQW_R2(L, 2);                         \
-        case 3: IQW_R2(L, 3);                         \
-        case 4: IQW_R2(L, 4);                         \
-        case 5: IQW_R2(L, 5);                         \
-        case 6: IQW_R2(L, 6);                         \
-        case 7: IQW_R2(L, 7);                         \
-        default: return IQW_ERR_UNSUPPORTED;          \
-    }
-    switch (log2n) {
-        case 10: IQW_R2F(10)
-        case 11: IQW_R2F(11)
-        case 12: IQW_R2F(12)
-    }
-#undef IQW_R2F
-#undef IQW_R2
-    return IQW_ERR_UNSUPPORTED;
+    auto unsupported = [] { return IQW_ERR_UNSUPPORTED; };
+    return dispatch<10, 12>(log2n, [&](auto L) {
+        return dispatch<1, 7>(flags, [&](auto F) { return launch2p_reduce_flags<L, F>(a, n_parts, stream); }, unsupported);
+    }, unsupported);
 }
 
 int stft_variant() { return g_stft_variant.load(); }
@@ -641,12 +599,8 @@ bool stft_two_pass_wanted(int log2n) {
 }
 
 int launch_stft_two_pass(const StftArgs& a, int log2n, int mode, cudaStream_t stream) {
-    switch (log2n) {
-        case 10: return launch2p<10>(a, mode, stream);
-        case 11: return launch2p<11>(a, mode, stream);
-        case 12: return launch2p<12>(a, mode, stream);
-    }
-    return fail(IQW_ERR_UNSUPPORTED, "two-pass stft: nfft=%d", 1 << log2n);
+    return dispatch<10, 12>(log2n, [&](auto L) { return launch2p<L>(a, mode, stream); },
+                            [&] { return fail(IQW_ERR_UNSUPPORTED, "two-pass stft: nfft=%d", 1 << log2n); });
 }
 
 }  // namespace iqw

@@ -28,9 +28,6 @@
 //     (st.shared::cluster into the readers' CTA): 20 % / 15 % of the HBM peak at nfft 32768 / 65536 with 256
 //     threads per CTA, 17 % / 13 % with three 128-thread CTAs per SM -- remote shared-memory stores sustain only
 //     ~20 B/clk per SM, an order of magnitude below the L2 path.
-#include <mutex>
-#include <map>
-#include <utility>
 #include "iqw_stft.cuh"
 
 namespace iqw {
@@ -308,31 +305,14 @@ __global__ void twiddle3p_init_kernel(float2* tw) {
     }
 }
 
-static std::mutex g_tw3_mutex;
-static std::map<int, float2*> g_tw3_cache;
-
-static int get_twiddles3p(cudaStream_t stream, const float2** out) {
-    int dev = 0;
-    IQW_CUDA_OK(cudaGetDevice(&dev));
-    std::lock_guard<std::mutex> lock(g_tw3_mutex);
-    auto it = g_tw3_cache.find(dev);
-    if (it == g_tw3_cache.end()) {
-        float2* d = nullptr;
-        IQW_CUDA_OK(cudaMalloc(&d, sizeof(float2) * 14 * 64));
-        twiddle3p_init_kernel<<<4, 256, 0, stream>>>(d);
-        IQW_CUDA_OK(cudaGetLastError());
-        IQW_CUDA_OK(cudaStreamSynchronize(stream));
-        it = g_tw3_cache.emplace(dev, d).first;
-    }
-    *out = it->second;
-    return IQW_OK;
-}
-
 template <int LOG2N, int MODE>
 static int launch3p_mode(StftArgs a, void* ws, size_t ws_bytes, cudaStream_t stream) {
     using C = P3Cfg<LOG2N>;
     auto kern = stft3p_kernel<LOG2N, MODE>;
-    if (int rc = get_twiddles3p(stream, &a.twiddle)) return rc;
+    if (int rc = device_table(kThreePassTwiddles, 0, 14 * 64,
+                              [](float2* d, int, cudaStream_t s) { twiddle3p_init_kernel<<<4, 256, 0, s>>>(d); }, stream,
+                              &a.twiddle))
+        return rc;
     IQW_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
     int sms = 0;
     if (int rc = device_sm_count(&sms)) return rc;
@@ -371,16 +351,6 @@ static int launch3p_mode(StftArgs a, void* ws, size_t ws_bytes, cudaStream_t str
     return IQW_OK;
 }
 
-template <int LOG2N>
-static int launch3p(const StftArgs& a, int mode, void* ws, size_t ws_bytes, cudaStream_t s) {
-    switch (mode) {
-        case IQW_STFT_COMPLEX: return launch3p_mode<LOG2N, IQW_STFT_COMPLEX>(a, ws, ws_bytes, s);
-        case IQW_STFT_POWER: return launch3p_mode<LOG2N, IQW_STFT_POWER>(a, ws, ws_bytes, s);
-        case IQW_STFT_DB: return launch3p_mode<LOG2N, IQW_STFT_DB>(a, ws, ws_bytes, s);
-    }
-    return fail(IQW_ERR_INVALID, "unknown stft mode %d", mode);
-}
-
 // a bulk copy needs 16-byte aligned source addresses: every frame start of every channel
 bool stft_three_pass_cluster_ok(const StftArgs& a, int log2n) {
     if (log2n < 13 || log2n > 16) return false;
@@ -399,13 +369,10 @@ size_t stft_three_pass_scratch_bytes(int log2n, long long n_channels, long long 
 }
 
 int launch_stft_three_pass_cluster(const StftArgs& a, int log2n, int mode, void* ws, size_t ws_bytes, cudaStream_t stream) {
-    switch (log2n) {
-        case 13: return launch3p<13>(a, mode, ws, ws_bytes, stream);
-        case 14: return launch3p<14>(a, mode, ws, ws_bytes, stream);
-        case 15: return launch3p<15>(a, mode, ws, ws_bytes, stream);
-        case 16: return launch3p<16>(a, mode, ws, ws_bytes, stream);
-    }
-    return fail(IQW_ERR_UNSUPPORTED, "cluster stft: nfft=%d", 1 << log2n);
+    return dispatch<13, 16>(
+        log2n,
+        [&](auto L) { return dispatch_stft_mode(mode, [&](auto M) { return launch3p_mode<L, M>(a, ws, ws_bytes, stream); }); },
+        [&] { return fail(IQW_ERR_UNSUPPORTED, "cluster stft: nfft=%d", 1 << log2n); });
 }
 
 }  // namespace iqw

@@ -121,28 +121,14 @@ static int launch_blue_mode(BlueArgs a, cudaStream_t stream) {
     using C = StftCfg<LOG2M>;
     auto kern = bluestein_kernel<LOG2M, MODE>;
     if (int rc = get_twiddles(LOG2M, stream, &a.twiddle)) return rc;
-    IQW_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-    int sms = 0, per_sm = 0;
-    if (int rc = device_sm_count(&sms)) return rc;
-    IQW_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, C::THREADS, C::SMEM));
-    if (per_sm < 1) return fail(IQW_ERR_CUDA, "bluestein kernel M=%d does not fit on an SM", C::N);
+    long long grid = 0;
+    if (int rc = resident_ctas(kern, C::THREADS, C::SMEM, "bluestein kernel", &grid)) return rc;
     a.groups_per_ch = (a.n_frames + C::FPC - 1) / C::FPC;
     a.n_groups = a.groups_per_ch * a.n_channels;
-    long long grid = (long long)sms * per_sm;
     if (grid > a.n_groups) grid = a.n_groups;
     { IQW_PROFILE("stft_bluestein_kernel", stream); kern<<<(unsigned)grid, C::THREADS, C::SMEM, stream>>>(a); }
     IQW_CUDA_OK(cudaGetLastError());
     return IQW_OK;
-}
-
-template <int LOG2M>
-static int launch_blue(const BlueArgs& a, int mode, cudaStream_t s) {
-    switch (mode) {
-        case IQW_STFT_COMPLEX: return launch_blue_mode<LOG2M, IQW_STFT_COMPLEX>(a, s);
-        case IQW_STFT_POWER: return launch_blue_mode<LOG2M, IQW_STFT_POWER>(a, s);
-        case IQW_STFT_DB: return launch_blue_mode<LOG2M, IQW_STFT_DB>(a, s);
-    }
-    return fail(IQW_ERR_INVALID, "unknown stft mode %d", mode);
 }
 
 // ---- composed path for longer frames: three elementwise kernels around two calls of the large FFT ----
@@ -195,10 +181,8 @@ extern "C" int iqw_stft_bluestein_c64(const void* d_x, int64_t n_channels, int64
     iqw::DeviceGuard _dev_guard(d_x);
     if (!d_x || !d_pre || !d_bh || !d_post || !d_out) return fail(IQW_ERR_INVALID, "null pointer argument");
     if (nfft < 2) return fail(IQW_ERR_INVALID, "nfft=%d", nfft);
-    if (m < 2 || (m & (m - 1)) || m < 2 * nfft - 1)
-        return fail(IQW_ERR_INVALID, "m=%d must be a power of two >= 2*nfft - 1", m);
-    int log2m = 0;
-    while ((1 << log2m) < m) ++log2m;
+    const int log2m = log2_exact(m);
+    if (log2m < 1 || m < 2 * nfft - 1) return fail(IQW_ERR_INVALID, "m=%d must be a power of two >= 2*nfft - 1", m);
     if (log2m < 4 || log2m > 13)
         return fail(IQW_ERR_UNSUPPORTED, "iqw_stft_bluestein_c64: convolution length %d outside 16..8192 (nfft <= 4096)", m);
     if (hop < 1) return fail(IQW_ERR_INVALID, "hop=%lld must be >= 1", (long long)hop);
@@ -224,19 +208,9 @@ extern "C" int iqw_stft_bluestein_c64(const void* d_x, int64_t n_channels, int64
     a.out = d_out;
     a.out_ch_stride = out_channel_stride;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    switch (log2m) {
-        case 4: return launch_blue<4>(a, mode, s);
-        case 5: return launch_blue<5>(a, mode, s);
-        case 6: return launch_blue<6>(a, mode, s);
-        case 7: return launch_blue<7>(a, mode, s);
-        case 8: return launch_blue<8>(a, mode, s);
-        case 9: return launch_blue<9>(a, mode, s);
-        case 10: return launch_blue<10>(a, mode, s);
-        case 11: return launch_blue<11>(a, mode, s);
-        case 12: return launch_blue<12>(a, mode, s);
-        case 13: return launch_blue<13>(a, mode, s);
-    }
-    return fail(IQW_ERR_UNSUPPORTED, "m=%d", m);
+    return dispatch<4, 13>(
+        log2m, [&](auto L) { return dispatch_stft_mode(mode, [&](auto M) { return launch_blue_mode<L, M>(a, s); }); },
+        [&] { return fail(IQW_ERR_UNSUPPORTED, "m=%d", m); });
 }
 
 // the three elementwise steps of the composed path (python drives the two FFT calls between them)
@@ -276,12 +250,9 @@ extern "C" int iqw_bluestein_post_c64(const void* d_a, const void* d_post, int32
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const float2* a = static_cast<const float2*>(d_a);
     const float2* post = static_cast<const float2*>(d_post);
-    switch (mode) {
-        case IQW_STFT_COMPLEX: blue_post_kernel<IQW_STFT_COMPLEX><<<sms * 8, 256, 0, s>>>(a, post, m, n_frames, bin_lo, bin_hi, eps, d_out); break;
-        case IQW_STFT_POWER: blue_post_kernel<IQW_STFT_POWER><<<sms * 8, 256, 0, s>>>(a, post, m, n_frames, bin_lo, bin_hi, eps, d_out); break;
-        case IQW_STFT_DB: blue_post_kernel<IQW_STFT_DB><<<sms * 8, 256, 0, s>>>(a, post, m, n_frames, bin_lo, bin_hi, eps, d_out); break;
-        default: return fail(IQW_ERR_INVALID, "unknown stft mode %d", mode);
-    }
-    IQW_CUDA_OK(cudaGetLastError());
-    return IQW_OK;
+    return dispatch_stft_mode(mode, [&](auto M) -> int {
+        blue_post_kernel<M><<<sms * 8, 256, 0, s>>>(a, post, m, n_frames, bin_lo, bin_hi, eps, d_out);
+        IQW_CUDA_OK(cudaGetLastError());
+        return IQW_OK;
+    });
 }

@@ -18,8 +18,6 @@
 // The scratch is written and read once (16*nfft/hop bytes per sample of extra HBM traffic); frames
 // are processed in chunks so that it never exceeds the scratch cap.
 #include <algorithm>
-#include <mutex>
-#include <map>
 #include <atomic>
 #include "iqw_stft.cuh"
 
@@ -278,26 +276,14 @@ __global__ void step_twiddle_kernel(float2* ta, float2* tb, int n1, long long n)
     }
 }
 
-static std::mutex g_step_mutex;
-static std::map<std::pair<int, int>, float2*> g_step_cache;
-
 static int get_step_twiddles(int log2n, cudaStream_t stream, const float2** ta, const float2** tb) {
-    int dev = 0;
-    IQW_CUDA_OK(cudaGetDevice(&dev));
-    std::lock_guard<std::mutex> lock(g_step_mutex);
-    auto key = std::make_pair(dev, log2n);
-    auto it = g_step_cache.find(key);
     const int n1 = 1 << (log2n - kLog2N2);
-    if (it == g_step_cache.end()) {
-        float2* d = nullptr;
-        IQW_CUDA_OK(cudaMalloc(&d, sizeof(float2) * (n1 + kN2)));
-        step_twiddle_kernel<<<(std::max(n1, kN2) + 255) / 256, 256, 0, stream>>>(d, d + n1, n1, 1ll << log2n);
-        IQW_CUDA_OK(cudaGetLastError());
-        IQW_CUDA_OK(cudaStreamSynchronize(stream));
-        it = g_step_cache.emplace(key, d).first;
-    }
-    *ta = it->second;
-    *tb = it->second + n1;
+    auto init = [](float2* d, int log2n, cudaStream_t s) {
+        const int n1 = 1 << (log2n - kLog2N2);
+        step_twiddle_kernel<<<(std::max(n1, kN2) + 255) / 256, 256, 0, s>>>(d, d + n1, n1, 1ll << log2n);
+    };
+    if (int rc = device_table(kStepTwiddles, log2n, n1 + kN2, init, stream, ta)) return rc;
+    *tb = *ta + n1;
     return IQW_OK;
 }
 
@@ -311,15 +297,12 @@ size_t stft_large_workspace_bytes(int log2n, long long n_channels, long long n_f
 }
 
 template <int L1>
-static int launch_columns(const LargeArgs& g, int sms, cudaStream_t s) {
+static int launch_columns(const LargeArgs& g, cudaStream_t s) {
     using C = ColCfg<L1>;
     auto kern = columns_kernel<L1>;
-    IQW_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-    int per_sm = 0;
-    IQW_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, C::THREADS, C::SMEM));
-    if (per_sm < 1) return fail(IQW_ERR_CUDA, "columns kernel does not fit on an SM");
+    long long grid = 0;
+    if (int rc = resident_ctas(kern, C::THREADS, C::SMEM, "columns kernel", &grid)) return rc;
     const long long items = (g.gf1 - g.gf0) * (kN2 / kCols);
-    long long grid = (long long)sms * per_sm;
     if (grid > items) grid = items;
     { IQW_PROFILE("stft_columns", s); kern<<<(unsigned)grid, C::THREADS, C::SMEM, s>>>(g); }
     IQW_CUDA_OK(cudaGetLastError());
@@ -327,14 +310,11 @@ static int launch_columns(const LargeArgs& g, int sms, cudaStream_t s) {
 }
 
 template <int MODE>
-static int launch_rows(const LargeArgs& g, int log2n1, int sms, cudaStream_t s) {
+static int launch_rows(const LargeArgs& g, int log2n1, cudaStream_t s) {
     auto kern = rows_kernel<MODE>;
-    IQW_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRowSmem));
-    int per_sm = 0;
-    IQW_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kRowThreads, kRowSmem));
-    if (per_sm < 1) return fail(IQW_ERR_CUDA, "rows kernel does not fit on an SM");
+    long long grid = 0;
+    if (int rc = resident_ctas(kern, kRowThreads, kRowSmem, "rows kernel", &grid)) return rc;
     const long long items = (g.gf1 - g.gf0) * ((1 << log2n1) / kCols);
-    long long grid = (long long)sms * per_sm;
     if (grid > items) grid = items;
     { IQW_PROFILE("stft_rows", s); kern<<<(unsigned)grid, kRowThreads, kRowSmem, s>>>(g, log2n1); }
     IQW_CUDA_OK(cudaGetLastError());
@@ -349,8 +329,6 @@ int launch_stft_large(const StftArgs& a, int log2n, int mode, void* workspace, s
         return fail(IQW_ERR_WORKSPACE, "nfft=%d needs a workspace of at least %zu bytes (iqw_stft_workspace_bytes)",
                     1 << log2n, frame_bytes);
     if (((uintptr_t)workspace & 15) != 0) return fail(IQW_ERR_INVALID, "workspace not 16-byte aligned");
-    int sms = 0;
-    if (int rc = device_sm_count(&sms)) return rc;
 
     LargeArgs g{};
     g.a = a;
@@ -368,22 +346,11 @@ int launch_stft_large(const StftArgs& a, int log2n, int mode, void* workspace, s
         g.gf0 = gf0;
         g.gf1 = gf0 + chunk < total ? gf0 + chunk : total;
         g.a.twiddle = tw_cols;
-        int rc = IQW_OK;
-        switch (log2n1) {
-            case 6: rc = launch_columns<6>(g, sms, stream); break;
-            case 7: rc = launch_columns<7>(g, sms, stream); break;
-            case 8: rc = launch_columns<8>(g, sms, stream); break;
-            default: return fail(IQW_ERR_UNSUPPORTED, "nfft=%d", 1 << log2n);
-        }
-        if (rc) return rc;
+        if (int rc = dispatch<6, 8>(log2n1, [&](auto L1) { return launch_columns<L1>(g, stream); },
+                                    [&] { return fail(IQW_ERR_UNSUPPORTED, "nfft=%d", 1 << log2n); }))
+            return rc;
         g.a.twiddle = tw_rows;
-        switch (mode) {
-            case IQW_STFT_COMPLEX: rc = launch_rows<IQW_STFT_COMPLEX>(g, log2n1, sms, stream); break;
-            case IQW_STFT_POWER: rc = launch_rows<IQW_STFT_POWER>(g, log2n1, sms, stream); break;
-            case IQW_STFT_DB: rc = launch_rows<IQW_STFT_DB>(g, log2n1, sms, stream); break;
-            default: return fail(IQW_ERR_INVALID, "unknown stft mode %d", mode);
-        }
-        if (rc) return rc;
+        if (int rc = dispatch_stft_mode(mode, [&](auto M) { return launch_rows<M>(g, log2n1, stream); })) return rc;
     }
     return IQW_OK;
 }
