@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define IQW_ABI_VERSION 11
+#define IQW_ABI_VERSION 12
 
 typedef enum iqw_status {
     IQW_OK = 0,
@@ -334,6 +334,38 @@ int iqw_pfb_channelize_c64(const void* d_x, int64_t n_channels, int64_t n_in, in
                            int64_t x_first, const void* d_taps, int32_t n_taps, int32_t nfft, int32_t hop,
                            int64_t frame_first, int64_t n_frames, void* d_out, int64_t out_channel_stride,
                            void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Kernel 9: polyphase synthesis bank, the adjoint of kernel 8 with a real synthesis prototype g of n_taps = Lg
+ * taps: recombines nfft = K channels of frame-major complex64 frames into one complex64 row per channel.
+ *
+ *   xr[t] = sum_m sum_k g[t - m*hop] * y[m, k] * exp(+2 pi i (k - K/2) t / K),  0 <= t - m*hop < Lg,
+ *           0 <= t < (T - 1)*hop + Lg,  m a GLOBAL frame index, T = n_frames_total
+ *
+ * With g = h this is exactly the adjoint of iqw_pfb_channelize_c64.  Two kernels: the first unrotates each
+ * frame with kernel 8's W_K table and writes u_m = K * IFFT_K to the workspace, the second sums every output
+ * from the frames that cover it, in ascending m.
+ *
+ *   d_y           (n_channels, n_frames, nfft) complex64, frame-major, channel stride y_channel_stride
+ *                 elements; holds GLOBAL frames [frame_first, frame_first + n_frames) of n_frames_total
+ *   d_taps        the folded, sign-applied float32 table of g, as for iqw_pfb_channelize_c64
+ *                 (python: iqwaveform_b200._plan.pfb_taps)
+ *   nfft          K, a power of two in 16..8192 (else IQW_ERR_UNSUPPORTED)
+ *   n_taps        Lg >= 1; P <= 16 and Lg <= 32768 are built (else IQW_ERR_UNSUPPORTED)
+ *   hop           frame step, 1 <= hop <= nfft (else IQW_ERR_INVALID)
+ *   out_first     global index of the first output; the call writes outputs [out_first, out_first + n_out)
+ *                 to d_out (n_channels, n_out) complex64, channel stride out_channel_stride elements.  Every
+ *                 frame those outputs need must be among the call's frames, and the outputs must lie before
+ *                 (T - 1)*hop + Lg (else IQW_ERR_INVALID)
+ *   d_workspace   >= iqw_pfb_synthesize_workspace_bytes(n_channels, n_frames, nfft) bytes (the size of d_y),
+ *                 16-byte aligned (else IQW_ERR_INVALID)
+ * An output's bits depend only on the frames that cover it, their global indices and the taps, so time
+ * shards concatenate to the bits of one call. */
+size_t iqw_pfb_synthesize_workspace_bytes(int64_t n_channels, int64_t n_frames, int32_t nfft);
+int iqw_pfb_synthesize_c64(const void* d_y, int64_t n_channels, int64_t n_frames, int64_t y_channel_stride,
+                           int64_t frame_first, int64_t n_frames_total, const void* d_taps, int32_t n_taps,
+                           int32_t nfft, int32_t hop, int64_t out_first, int64_t n_out, void* d_out,
+                           int64_t out_channel_stride, void* d_workspace, size_t workspace_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Exact order statistics of a float32 matrix whose ROWS are spread over several GPUs (the

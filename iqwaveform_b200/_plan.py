@@ -389,6 +389,11 @@ def pfb_frame_count(n_samples: int, n_taps: int, hop: int) -> int:
     return (n_samples - n_taps) // hop + 1
 
 
+def pfb_synth_len(n_frames: int, n_taps: int, hop: int) -> int:
+    """samples of pfb_synthesize from n_frames frames and an n_taps synthesis prototype: (T - 1) * hop + Lg"""
+    return (n_frames - 1) * hop + n_taps
+
+
 def pfb_taps(h: np.ndarray, nfft: int) -> np.ndarray:
     """the folded, sign-applied float32 tap table of iqw_pfb_channelize_c64: h rounded once to float32,
     zero-padded to P = ceil(L / nfft) rows of nfft, row p holding (-1)^r h[r + p*nfft]"""

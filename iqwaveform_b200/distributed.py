@@ -16,6 +16,8 @@ The path shards without any collective on the data path, with one exception (the
   the discard D (not M - 1) before them and the rest of its last block after them
 * pfb_channelize frames are independent         -> `pfb_shard` (pfb_channelize): rank r owns frames
   [f0, f1) and reads [f0*hop, (f1 - 1)*hop + L), a halo of L - hop samples
+* pfb_synthesize outputs are independent         -> `pfb_synth_shard` (pfb_synthesize): rank r owns outputs
+  [o0, o1) and reads the frames that cover them, a halo of about Lg / hop - 1 frames
 * exact quantiles of ONE capture split in time -> `persistence_spectrum_time_sharded`: the only
   real exchange step of the path -- per-bin digit counts of a radix select are all_reduced
   (`select_order_statistics`; kernels in csrc/iqw_rowsplit.cu)
@@ -35,7 +37,7 @@ __all__ = ['channel_shard', 'frame_shard', 'bin_shard', 'gather_rows', 'persiste
            'persistence_spectrum_time_sharded', 'select_order_statistics', 'CudaShardOps', 'ThreadGroup',
            'bind_to_gpu_numa_node', 'spectrogram_time_sharded', 'iq_to_bin_power_sharded', 'upfirdn_shard',
            'upfirdn_time_sharded', 'oaconvolve_shard', 'oaconvolve_time_sharded', 'pfb_shard',
-           'pfb_channelize_time_sharded']
+           'pfb_channelize_time_sharded', 'pfb_synth_shard', 'pfb_synthesize_time_sharded']
 
 
 def _split(n: int, world: int, rank: int) -> tuple[int, int]:
@@ -701,3 +703,62 @@ def pfb_channelize_time_sharded(x_halo, h, nchannels, hop=None, *, n_samples: in
         return y
     sizes = [(lambda s: s.frame1 - s.frame0)(pfb_shard(n_samples, L, K, hop, world, r)) for r in range(world)]
     return gather_rows(y, sizes, 0, group)
+
+
+class PfbSynthShard(NamedTuple):
+    out0: int       # first output of this rank
+    out1: int       # one past its last output
+    frame0: int     # first frame it reads
+    frame1: int     # one past the last frame it reads (includes the halo)
+    n_out: int      # outputs of the whole capture
+
+
+def pfb_synth_shard(n_frames: int, n_taps: int, nchannels: int, hop: int | None, world: int,
+                    rank: int) -> PfbSynthShard:
+    """time-axis shard of pfb_synthesize(y, g, hop) for n_frames frames and an n_taps synthesis prototype: the
+    (T - 1) * hop + Lg outputs are split evenly, and rank r reads the frames [max(0, ceil((o0 - Lg + 1) / hop)),
+    min(T, floor((o1 - 1) / hop) + 1)) that cover its outputs [o0, o1) (an empty range where they all fall in a
+    gap between frames, Lg < hop).  An output sums the same terms in the same order wherever it is computed, so
+    the shards' concatenation is bitwise the single-GPU result."""
+    from . import _plan
+    hop = nchannels if hop is None else hop
+    if n_taps < 1 or not 1 <= hop <= nchannels or n_frames < 1:
+        raise ValueError(f'pfb synthesis shards need n_taps >= 1, 1 <= hop <= nchannels and n_frames >= 1 '
+                         f'(got {n_taps}, {hop}, {n_frames})')
+    n_out = _plan.pfb_synth_len(n_frames, n_taps, hop)
+    o0, o1 = _split(n_out, world, rank)
+    f0 = max(0, -(-(o0 - n_taps + 1) // hop))
+    f1 = min(n_frames, (o1 - 1) // hop + 1) if o1 > o0 else f0
+    f0 = min(f0, n_frames)
+    return PfbSynthShard(o0, o1, f0, max(f0, f1), n_out)
+
+
+def pfb_synthesize_time_sharded(y_halo, g, hop=None, *, n_frames: int, group=None, compute: Callable | None = None,
+                                gather: bool = False):
+    """time-sharded pfb_synthesize(y, g, hop) of n_frames frame-major frames y (T, K) complex64: `y_halo` holds
+    this rank's frames [shard.frame0, shard.frame1) of `pfb_synth_shard` (halo included) as a (frames, K)
+    array.  Returns this rank's outputs [out0, out1) or, with gather=True, all outputs on every rank; the
+    concatenation is bitwise the single-GPU `pfb_synthesize`.
+    `compute(y_halo, taps, n_taps, hop, frame_first=, n_frames_total=, out_first=, n_out=)` defaults to the CUDA
+    kernels."""
+    from . import fourier
+    if y_halo.ndim != 2:
+        raise ValueError(f'pfb_synthesize_time_sharded: y_halo must be (frames, nchannels), got {tuple(y_halo.shape)}')
+    taps, Lg, K, hop = fourier._pfb_args(g, y_halo.shape[1], hop, what='pfb_synthesize', name='g')
+    world, rank = _world(group)
+    sh = pfb_synth_shard(n_frames, Lg, K, hop, world, rank)
+    if y_halo.shape[0] != sh.frame1 - sh.frame0:
+        raise ValueError(f'rank {rank} expects a shard of {sh.frame1 - sh.frame0} frames, got {tuple(y_halo.shape)}')
+    kw = dict(frame_first=sh.frame0, n_frames_total=n_frames, out_first=sh.out0, n_out=sh.out1 - sh.out0)
+    if compute is None:
+        from . import _arrays
+        yd, _ = _arrays.to_device(y_halo)
+        if yd.dtype != torch.complex64:
+            raise NotImplementedError(f'pfb_synthesize: only complex64 frames are built (got {yd.dtype})')
+        x = fourier._pfb_synth_device(yd.reshape(1, -1, K), taps, Lg, hop, **kw)[0]
+    else:
+        x = torch.as_tensor(compute(y_halo, taps, Lg, hop, **kw))
+    if not gather or world == 1:
+        return x
+    sizes = [(lambda s: s.out1 - s.out0)(pfb_synth_shard(n_frames, Lg, K, hop, world, r)) for r in range(world)]
+    return gather_rows(x, sizes, 0, group)
