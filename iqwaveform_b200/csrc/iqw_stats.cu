@@ -13,7 +13,7 @@
 // level; per column the state is a short ordered list of disjoint key INTERVALS, each known to
 // contain a contiguous group of the target ranks, with the exact number of keys below it:
 //
-// EXACT PIPELINE (any row set):
+// EXACT PIPELINE (rows < 16384; every pass reads all rows):
 //   range   : min/max key of ~2k rows per column  -> bucket map of that column
 //   L0      : 256-bucket histogram of every element (bucket 0 / 255 catch keys outside the range
 //             seen by `range`, so counts are exact whatever it missed)
@@ -116,8 +116,8 @@ struct BracketPlan {
     unsigned int cap_sum;                        // keys a (row split, column) candidate list holds
 };
 
-// rows visited by a streaming pass: all of them (step == 1) or one pseudo-random row out of every
-// `step` consecutive rows (a stratified sample; the jitter defeats periodic captures)
+// the row sample of sample_brackets: one pseudo-random row out of every `step` consecutive rows
+// (a stratified sample; the jitter defeats periodic captures)
 struct RowMap {
     long long n;       // rows visited
     long long step;
@@ -222,52 +222,33 @@ static size_t carve_work(void* base, int64_t cols, int64_t splits, int64_t cap_s
 }
 
 // ---------------------------------------------------------------------------------------------
-// streaming skeleton: thread `col` visits rows i0..i1 of the row map, kUnroll loads in flight
+// streaming skeleton: thread `col` visits rows i0..i1, kUnroll loads in flight
 // ---------------------------------------------------------------------------------------------
-template <bool SAMPLED, typename F>
+template <typename F>
 __device__ __forceinline__ void stream_column(const float* __restrict__ p, long long cols,
-                                              long long col, const RowMap& rm, long long i0,
-                                              long long i1, F&& visit) {
+                                              long long col, long long i0, long long i1, F&& visit) {
     long long i = i0;
-    if (!SAMPLED) {
-        const float* src = p + i0 * cols + col;
-        for (; i + kUnroll <= i1; i += kUnroll, src += (long long)kUnroll * cols) {
-            float f[kUnroll];
+    const float* src = p + i0 * cols + col;
+    for (; i + kUnroll <= i1; i += kUnroll, src += (long long)kUnroll * cols) {
+        float f[kUnroll];
 #pragma unroll
-            for (int u = 0; u < kUnroll; ++u) f[u] = __ldcs(src + (long long)u * cols);
+        for (int u = 0; u < kUnroll; ++u) f[u] = __ldcs(src + (long long)u * cols);
 #pragma unroll
-            for (int u = 0; u < kUnroll; ++u) visit(f[u]);
-        }
-        for (; i < i1; ++i, src += cols) visit(__ldcs(src));
-    } else {
-        for (; i + kUnroll <= i1; i += kUnroll) {
-            float f[kUnroll];
-#pragma unroll
-            for (int u = 0; u < kUnroll; ++u) f[u] = __ldg(p + map_row(rm, i + u) * cols + col);
-#pragma unroll
-            for (int u = 0; u < kUnroll; ++u) visit(f[u]);
-        }
-        for (; i < i1; ++i) visit(__ldg(p + map_row(rm, i) * cols + col));
+        for (int u = 0; u < kUnroll; ++u) visit(f[u]);
     }
+    for (; i < i1; ++i, src += cols) visit(__ldcs(src));
 }
 
-#define IQW_STREAM(SAMPLED_FLAG, ...)                                                      \
-    do {                                                                                   \
-        if (SAMPLED_FLAG) stream_column<true>(__VA_ARGS__);                                \
-        else stream_column<false>(__VA_ARGS__);                                            \
-    } while (0)
-
 // ---------------------------------------------------------------------------------------------
-// range: min / max key over ~2k of the visited rows
+// range: min / max key over ~2k of the rows
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(kBX)
-range_kernel(const float* __restrict__ p, long long cols, RowMap rm, long long stride, Work w) {
+range_kernel(const float* __restrict__ p, long long cols, long long rows, long long stride, Work w) {
     const long long col = (long long)blockIdx.x * kBX + threadIdx.x;
     if (col >= cols) return;
     uint32_t lo = 0xFFFFFFFFu, hi = 0u;
-    for (long long i = (long long)blockIdx.y * stride; i < rm.n; i += stride * gridDim.y) {
-        const long long r = rm.step == 1 ? i : map_row(rm, i);
-        const uint32_t k = float_to_key(__ldg(p + r * cols + col));
+    for (long long i = (long long)blockIdx.y * stride; i < rows; i += stride * gridDim.y) {
+        const uint32_t k = float_to_key(__ldg(p + i * cols + col));
         lo = min(lo, k);
         hi = max(hi, k);
     }
@@ -315,11 +296,11 @@ struct Named {
 };
 
 // ---------------------------------------------------------------------------------------------
-// L0: private 256-bucket histogram per column (+ named statistics when NAMED)
+// L0: private 256-bucket histogram per column + named statistics
 // ---------------------------------------------------------------------------------------------
-template <bool NAMED, bool WANT_SUM, bool TO_DB>
+template <bool WANT_SUM, bool TO_DB>
 __global__ void __launch_bounds__(kBX)
-l0_kernel(const float* __restrict__ p, long long cols, RowMap rm, long long rows_per_split,
+l0_kernel(const float* __restrict__ p, long long cols, long long rows, long long rows_per_split,
           float eps, Work w) {
     extern __shared__ uint16_t hist[];   // [kNB0][kBX]
     for (int i = threadIdx.x; i < kNB0 * kBX; i += kBX) hist[i] = 0;
@@ -331,22 +312,22 @@ l0_kernel(const float* __restrict__ p, long long cols, RowMap rm, long long rows
     const uint32_t s = l0_shift(lo, hi);
     uint16_t* h = hist + threadIdx.x;
     const long long i0 = (long long)blockIdx.y * rows_per_split;
-    const long long i1 = min(rm.n, i0 + rows_per_split);
+    const long long i1 = min(rows, i0 + rows_per_split);
     Named<true, WANT_SUM, TO_DB> named;
 
     auto visit = [&](float f) {
         const uint32_t k = float_to_key(f);
-        if (NAMED) named.add(f, k, eps);
+        named.add(f, k, eps);
         h[l0_bucket(k, lo, hi, s) * kBX] += 1;
     };
-    IQW_STREAM(rm.step != 1, p, cols, col, rm, i0, i1, visit);
+    stream_column(p, cols, col, i0, i1, visit);
 
     uint32_t* g = w.hist0 + col * kNB0;
     for (int b = 0; b < kNB0; ++b) {
         const uint32_t c = h[b * kBX];
         if (c) atomicAdd(g + b, c);
     }
-    if (NAMED) named.flush(w, col);
+    named.flush(w, col);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -612,11 +593,11 @@ struct IvRegs {
 // refine: 32 sub-buckets per pending interval, private counters [interval*32+sub][thread]
 template <int M>
 __device__ __forceinline__ void refine_body(unsigned bx, unsigned by, unsigned gdx, const float* __restrict__ p, long long cols,
-                                            RowMap rm, long long rows_per_split, const Work& w, uint16_t* hist /* [M*32][kBX] */) {
+                                            long long rows, long long rows_per_split, const Work& w, uint16_t* hist /* [M*32][kBX] */) {
     const int t = threadIdx.x;
     const long long col_tiles = (cols + kBX - 1) / kBX;
     const long long i0 = (long long)by * rows_per_split;
-    const long long i1 = min(rm.n, i0 + rows_per_split);
+    const long long i1 = min(rows, i0 + rows_per_split);
     // a CTA owns the row range of `by` and walks column tiles bx, + gdx, ...;
     // tiles without a pending interval cost one look at their interval lists.  (After the long
     // path only a few tiles are ever pending, so its launch uses few tile slots and many row
@@ -636,7 +617,7 @@ __device__ __forceinline__ void refine_body(unsigned bx, unsigned by, unsigned g
                 const int v = iv.find(k, kl, kh, sh);
                 if (v >= 0 && k <= kh && sh < 32u) hist[(v * kNSub + ((k - kl) >> sh)) * kBX + t] += 1;
             };
-            IQW_STREAM(rm.step != 1, p, cols, col, rm, i0, i1, visit);
+            stream_column(p, cols, col, i0, i1, visit);
 
             uint32_t* g = w.hist1 + col * (kMaxRanks * kNSub);
 #pragma unroll
@@ -655,11 +636,11 @@ __device__ __forceinline__ void refine_body(unsigned bx, unsigned by, unsigned g
 // refine: 32 sub-buckets per pending interval, private counters [interval*32+sub][thread]
 template <int M>
 __global__ void __launch_bounds__(kBX)
-refine_kernel(const float* __restrict__ p, long long cols, RowMap rm, long long rows_per_split,
+refine_kernel(const float* __restrict__ p, long long cols, long long rows, long long rows_per_split,
               Work w) {
     if (*w.pending == 0) return;
     extern __shared__ uint16_t hist[];   // [M*32][kBX]
-    refine_body<M>(blockIdx.x, blockIdx.y, gridDim.x, p, cols, rm, rows_per_split, w, hist);
+    refine_body<M>(blockIdx.x, blockIdx.y, gridDim.x, p, cols, rows, rows_per_split, w, hist);
 }
 
 // bracket pass (long-column path): the ONE read of all rows.  A thread owns a column; its M
@@ -939,10 +920,10 @@ bracket_pass_kernel(const float* __restrict__ p, long long cols, long long rows,
 
 template <int M>
 __device__ __forceinline__ void collect_body(unsigned bx, unsigned by, unsigned gdx, const float* __restrict__ p,
-                                             long long cols, RowMap rm, long long rows_per_split, const Work& w) {
+                                             long long cols, long long rows, long long rows_per_split, const Work& w) {
     const long long col_tiles = (cols + kBX - 1) / kBX;
     const long long i0 = (long long)by * rows_per_split;
-    const long long i1 = min(rm.n, i0 + rows_per_split);
+    const long long i1 = min(rows, i0 + rows_per_split);
     for (long long tile = bx; tile < col_tiles; tile += gdx) {     // see refine_body
         const long long col = tile * kBX + threadIdx.x;
         int active = 0;
@@ -960,16 +941,16 @@ __device__ __forceinline__ void collect_body(unsigned bx, unsigned by, unsigned 
                 if (pos < (uint32_t)kCap) w.cand[x * kCap + pos] = k;
             }
         };
-        IQW_STREAM(rm.step != 1, p, cols, col, rm, i0, i1, visit);
+        stream_column(p, cols, col, i0, i1, visit);
     }
 }
 
 template <int M>
 __global__ void __launch_bounds__(kBX)
-collect_kernel(const float* __restrict__ p, long long cols, RowMap rm, long long rows_per_split,
+collect_kernel(const float* __restrict__ p, long long cols, long long rows, long long rows_per_split,
                Work w) {
     if (w.pending[1] == 0) return;
-    collect_body<M>(blockIdx.x, blockIdx.y, gridDim.x, p, cols, rm, rows_per_split, w);
+    collect_body<M>(blockIdx.x, blockIdx.y, gridDim.x, p, cols, rows, rows_per_split, w);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1632,7 +1613,6 @@ __global__ void finalize_kernel(long long rows, long long cols, StatPlan st, int
 struct TailArgs {
     const float* p;
     long long rows, cols;
-    RowMap rm;
     unsigned gx, gy;              // virtual grid of the refine / collect steps (tile slots x row splits)
     long long rows_per_split;
     RankPlan rp;
@@ -1657,7 +1637,7 @@ tail_kernel(TailArgs a) {
             // (virtual block vb = tile slot * row splits + row split: the row splits of a pending tile spread over ALL CTAs)
             if (open)
                 for (unsigned vb = blockIdx.x; vb < nvb; vb += gridDim.x)
-                    refine_body<M>(vb / a.gy, vb % a.gy, a.gx, a.p, a.cols, a.rm, a.rows_per_split, w,
+                    refine_body<M>(vb / a.gy, vb % a.gy, a.gx, a.p, a.cols, a.rows, a.rows_per_split, w,
                                    reinterpret_cast<uint16_t*>(tail_smem));
             grid.sync();
             if (open)
@@ -1667,7 +1647,7 @@ tail_kernel(TailArgs a) {
         }
         if (w.pending[1] != 0u) {                       // nobody writes it after the last scan step
             for (unsigned vb = blockIdx.x; vb < nvb; vb += gridDim.x)
-                collect_body<M>(vb / a.gy, vb % a.gy, a.gx, a.p, a.cols, a.rm, a.rows_per_split, w);
+                collect_body<M>(vb / a.gy, vb % a.gy, a.gx, a.p, a.cols, a.rows, a.rows_per_split, w);
             grid.sync();
             for (long long col = blockIdx.x; col < a.cols; col += gridDim.x) {
                 resolve_body(col, a.rp, w, reinterpret_cast<uint32_t*>(tail_smem));
@@ -1835,51 +1815,48 @@ struct Grid {
     long long rows_per_split;
 };
 
-static int plan_grid(long long n_rows, long long col_tiles, int sms, Grid* g) {
-    // time splits: enough CTAs to fill the machine a few times, < 65536 rows each (uint16 counters)
-    long long splits = (4ll * sms * 4 + col_tiles - 1) / col_tiles;
+// grid of the streaming passes: tile slots (at most `max_slots` column tiles; a CTA walks the tiles of its slot) x
+// row splits, enough CTAs to fill the machine `ctas_per_sm` times, < 65536 rows per split (uint16 counters)
+static int plan_grid(long long n_rows, long long col_tiles, long long max_slots, int ctas_per_sm, int sms, Grid* g) {
+    const long long slots = col_tiles < max_slots ? col_tiles : max_slots;
+    long long splits = ((long long)ctas_per_sm * sms + slots - 1) / slots;
     if (splits < 1) splits = 1;
     long long rps = (n_rows + splits - 1) / splits;
     if (rps > 65535) rps = 65535;
     if (rps < 4 * kUnroll) rps = 4 * kUnroll;
     splits = (n_rows + rps - 1) / rps;
     if (splits > 65535) return fail(IQW_ERR_UNSUPPORTED, "too many rows for the split grid");
-    g->grid = dim3((unsigned)col_tiles, (unsigned)splits);
+    g->grid = dim3((unsigned)slots, (unsigned)splits);
     g->rows_per_split = rps;
     return IQW_OK;
 }
 
+// the interval train: 7 x (refine, scan), collect, resolve; each kernel exits at once when nothing is open
 template <int M>
-static void launch_refine_levels(const Grid& g, cudaStream_t s, const float* p, long long cols,
-                                 RowMap rm, const RankPlan& rp, const Work& w, unsigned cblocks,
-                                 unsigned cthreads, const char* tag) {
-    static const char* const names[2][kRefineLevels] = {
-        {"stats_refine_1", "stats_refine_2", "stats_refine_3", "stats_refine_4", "stats_refine_5",
-         "stats_refine_6", "stats_refine_7"},
-        {"sample_refine_1", "sample_refine_2", "sample_refine_3", "sample_refine_4",
-         "sample_refine_5", "sample_refine_6", "sample_refine_7"}};
-    const int which = tag[1] == 'a' ? 1 : 0;   // "sample" vs "stats"
+static int launch_interval_train(const Grid& g, cudaStream_t s, const float* p, long long rows, long long cols,
+                                 const RankPlan& rp, const Work& w, unsigned cblocks, unsigned cthreads) {
+    static const char* const refine_names[kRefineLevels] = {"stats_refine_1", "stats_refine_2", "stats_refine_3",
+                                                            "stats_refine_4", "stats_refine_5", "stats_refine_6",
+                                                            "stats_refine_7"};
     const size_t smem = sizeof(uint16_t) * M * kNSub * kBX;
     cudaFuncSetAttribute(refine_kernel<M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     for (int level = 0; level < kRefineLevels; ++level) {
-        { IQW_PROFILE_FINE(names[which][level], s);
-          refine_kernel<M><<<g.grid, kBX, smem, s>>>(p, cols, rm, g.rows_per_split, w); }
-        { IQW_PROFILE_FINE(which ? "sample_scan" : "stats_scan", s);
+        { IQW_PROFILE_FINE(refine_names[level], s);
+          refine_kernel<M><<<g.grid, kBX, smem, s>>>(p, cols, rows, g.rows_per_split, w); }
+        { IQW_PROFILE_FINE("stats_scan", s);
           scan_refine_kernel<<<cblocks, cthreads, 0, s>>>(cols, rp, w); }
     }
+    { IQW_PROFILE_FINE("stats_collect", s);
+      collect_kernel<M><<<g.grid, kBX, 0, s>>>(p, cols, rows, g.rows_per_split, w); }
+    { IQW_PROFILE_FINE("stats_resolve", s);
+      resolve_kernel<<<(unsigned)cols, kResolveThreads, 0, s>>>(cols, rp, w); }
+    return IQW_OK;
 }
 
 template <int M>
-static void launch_collect(const Grid& g, cudaStream_t s, const float* p, long long cols, RowMap rm,
-                           const Work& w, const char* name) {
-    IQW_PROFILE_FINE(name, s);
-    collect_kernel<M><<<g.grid, kBX, 0, s>>>(p, cols, rm, g.rows_per_split, w);
-}
-
-template <int M>
-static void launch_bracket_pass(cudaStream_t s, const float* p, long long cols, long long rows,
-                                const LongPlan& lp, bool want_minmax, bool want_sum, bool to_dB, float eps,
-                                const Work& w) {
+static int launch_bracket_pass(cudaStream_t s, const float* p, long long cols, long long rows,
+                               const LongPlan& lp, bool want_minmax, bool want_sum, bool to_dB, float eps,
+                               const Work& w) {
     const dim3 grid((unsigned)((cols + kBX - 1) / kBX), (unsigned)lp.splits);
     IQW_PROFILE("stats_bracket_pass", s);
 #define IQW_BP(N) bracket_pass_kernel<M, N><<<grid, kBX, 0, s>>>(p, cols, rows, lp.rows_per_split, eps, lp.bp, w)
@@ -1893,6 +1870,7 @@ static void launch_bracket_pass(cudaStream_t s, const float* p, long long cols, 
         default: IQW_BP(7); break;
     }
 #undef IQW_BP
+    return IQW_OK;
 }
 
 // grid of the cooperative tail kernel: every CTA must be resident (a few per SM are plenty: its common case is
@@ -1935,63 +1913,52 @@ static int launch_select(cudaStream_t s, long long cols, const RankPlan& rp, con
     return IQW_OK;
 }
 
-#define IQW_DISPATCH_G(m, CALL)                  \
-    do {                                         \
-        if ((m) <= 1) { constexpr int M = 1; CALL; }        \
-        else if ((m) <= 2) { constexpr int M = 2; CALL; }   \
-        else if ((m) <= 4) { constexpr int M = 4; CALL; }   \
-        else { constexpr int M = 8; CALL; }                 \
-    } while (0)
+// Calls f(std::integral_constant<int, M>) with M, the register-array size of the interval and bracket kernels, the
+// smallest power of two >= n that is at least 2^LO (n <= 8 intervals or brackets)
+template <int LO, class F>
+static int dispatch_m(int n, F&& f) {
+    int l = LO;
+    while (l < 3 && (1 << l) < n) ++l;
+    return dispatch<LO, 3>(l, [&](auto L) { return f(std::integral_constant<int, 1 << decltype(L)::value>{}); },
+                           [] { return IQW_ERR_INVALID; });
+}
 
-#define IQW_DISPATCH_M(m, CALL)                  \
-    do {                                         \
-        if ((m) <= 2) { constexpr int M = 2; CALL; }        \
-        else if ((m) <= 4) { constexpr int M = 4; CALL; }   \
-        else { constexpr int M = 8; CALL; }                 \
-    } while (0)
-
-// exact pipeline on the rows of `rm`: leaves the key of every target rank in w.r_key
-static int run_exact(const float* p, long long cols, RowMap rm, const RankPlan& rp, bool named,
-                     bool want_sum, bool to_dB, float eps, const Work& w, int sms, cudaStream_t s,
-                     bool sample) {
+// exact pipeline on every row: leaves the key of every target rank in w.r_key
+static int run_exact(const float* p, long long rows, long long cols, const RankPlan& rp, bool want_sum, bool to_dB,
+                     float eps, const Work& w, int sms, cudaStream_t s) {
     const long long col_tiles = (cols + kBX - 1) / kBX;
     Grid g;
-    if (int rc = plan_grid(rm.n, col_tiles, sms, &g)) return rc;
+    if (int rc = plan_grid(rows, col_tiles, col_tiles, 16, sms, &g)) return rc;
     const unsigned cthreads = 128, cblocks = (unsigned)((cols + cthreads - 1) / cthreads);
 
-    long long stride = rm.n / 2048;
+    long long stride = rows / 2048;
     if (stride < 1) stride = 1;
-    long long rsplits = (rm.n + stride - 1) / stride / 64;
+    long long rsplits = (rows + stride - 1) / stride / 64;
     if (rsplits < 1) rsplits = 1;
     if (rsplits > 64) rsplits = 64;
     // (range, l0, scan0, 7 x (refine, scan), collect, resolve)
-    IQW_PROFILE_TRAIN(sample ? "sample_exact" : "stats_exact", s, rp.n_ranks > 0 ? 3 + 2 * kRefineLevels + 2 : 2);
-    { IQW_PROFILE_FINE(sample ? "sample_range" : "stats_range", s);
-      range_kernel<<<dim3((unsigned)col_tiles, (unsigned)rsplits), kBX, 0, s>>>(p, cols, rm, stride, w); }
+    IQW_PROFILE_TRAIN("stats_exact", s, rp.n_ranks > 0 ? 3 + 2 * kRefineLevels + 2 : 2);
+    { IQW_PROFILE_FINE("stats_range", s);
+      range_kernel<<<dim3((unsigned)col_tiles, (unsigned)rsplits), kBX, 0, s>>>(p, cols, rows, stride, w); }
 
-    const size_t l0_smem = sizeof(uint16_t) * kNB0 * kBX;
     {
-        IQW_PROFILE_FINE(sample ? "sample_l0" : "stats_l0", s);
-#define IQW_L0(A, B, C)                                                                              \
-    do {                                                                                             \
-        cudaFuncSetAttribute(l0_kernel<A, B, C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l0_smem); \
-        l0_kernel<A, B, C><<<g.grid, kBX, l0_smem, s>>>(p, cols, rm, g.rows_per_split, eps, w);       \
-    } while (0)
-        if (!named) IQW_L0(false, false, false);
-        else if (want_sum && to_dB) IQW_L0(true, true, true);
-        else if (want_sum) IQW_L0(true, true, false);
-        else IQW_L0(true, false, false);
-#undef IQW_L0
+        IQW_PROFILE_FINE("stats_l0", s);
+        const size_t smem = sizeof(uint16_t) * kNB0 * kBX;
+        auto l0 = [&](auto kernel) {
+            cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            kernel<<<g.grid, kBX, smem, s>>>(p, cols, rows, g.rows_per_split, eps, w);
+        };
+        if (want_sum && to_dB) l0(l0_kernel<true, true>);
+        else if (want_sum) l0(l0_kernel<true, false>);
+        else l0(l0_kernel<false, false>);
     }
     if (rp.n_ranks > 0) {
-        { IQW_PROFILE_FINE(sample ? "sample_scan" : "stats_scan", s);
+        { IQW_PROFILE_FINE("stats_scan", s);
           scan0_kernel<<<cblocks, cthreads, 0, s>>>(cols, rp, w); }
-        IQW_DISPATCH_M(rp.n_ranks, launch_refine_levels<M>(g, s, p, cols, rm, rp, w, cblocks, cthreads,
-                                                           sample ? "sample" : "stats"));
-        IQW_DISPATCH_M(rp.n_ranks, launch_collect<M>(g, s, p, cols, rm, w,
-                                                     sample ? "sample_collect" : "stats_collect"));
-        { IQW_PROFILE_FINE(sample ? "sample_resolve" : "stats_resolve", s);
-          resolve_kernel<<<(unsigned)cols, kResolveThreads, 0, s>>>(cols, rp, w); }
+        if (int rc = dispatch_m<1>(rp.n_ranks, [&](auto M) {
+                return launch_interval_train<M>(g, s, p, rows, cols, rp, w, cblocks, cthreads);
+            }))
+            return rc;
     }
     IQW_CUDA_OK(cudaGetLastError());
     return IQW_OK;
@@ -2078,7 +2045,6 @@ extern "C" int iqw_time_stats_f32(const float* d_p, int64_t n_channels, int64_t 
     if (int rc = device_sm_count(&sms)) return rc;
     const long long col_tiles = (n_cols + kBX - 1) / kBX;
     const unsigned cthreads = 128, cblocks = (unsigned)((n_cols + cthreads - 1) / cthreads);
-    RowMap full{n_rows, 1, 0u};
     if (sampled)
         IQW_CUDA_OK(cudaFuncSetAttribute(sample_brackets_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)kSampleSmem));
@@ -2089,44 +2055,36 @@ extern "C" int iqw_time_stats_f32(const float* d_p, int64_t n_channels, int64_t 
         { IQW_PROFILE_FINE("stats_init", s); if (int rc = reset_work(w, s)) return rc; }
 
         if (!sampled) {
-            if (int rc = run_exact(p, n_cols, full, rp, true, want_sum, to_dB != 0, eps, w, sms, s, false))
-                return rc;
+            if (int rc = run_exact(p, n_rows, n_cols, rp, want_sum, to_dB != 0, eps, w, sms, s)) return rc;
         } else {
             { IQW_PROFILE("stats_sample", s);
               sample_brackets_kernel<<<(unsigned)((n_cols + kSampleCols - 1) / kSampleCols), kSampleThreads,
                                        kSampleSmem, s>>>(p, n_cols, lp.sample, lp.bp, w); }
-            IQW_DISPATCH_G(lp.bp.n_groups, launch_bracket_pass<M>(s, p, n_cols, n_rows, lp, want_minmax, want_sum, to_dB != 0, eps, w));
+            if (int rc = dispatch_m<0>(lp.bp.n_groups, [&](auto M) {
+                    return launch_bracket_pass<M>(s, p, n_cols, n_rows, lp, want_minmax, want_sum, to_dB != 0, eps, w);
+                }))
+                return rc;
             { IQW_PROFILE("stats_scan", s);
               scan_brackets_kernel<<<cblocks, cthreads, 0, s>>>(n_cols, n_rows, rp, lp.bp.n_groups, w); }
-            IQW_DISPATCH_G(lp.bp.n_groups, if (int rc = launch_select<M>(s, n_cols, rp, lp, w)) return rc);
+            if (int rc = dispatch_m<0>(lp.bp.n_groups, [&](auto M) { return launch_select<M>(s, n_cols, rp, lp, w); }))
+                return rc;
             // whatever select could not settle from the lists (missed brackets, overflowed lists,
             // heavy ties) is refined from the matrix; these exit at once when nothing is open
             // few tile slots x many row splits: when one column misses, the whole GPU reads its tile
             Grid g;
-            {
-                const long long slots = col_tiles < 4 ? col_tiles : 4;
-                long long splits = (32ll * sms + slots - 1) / slots;
-                long long rps = (n_rows + splits - 1) / splits;
-                if (rps < 4 * kUnroll) rps = 4 * kUnroll;
-                if (rps > 65535) rps = 65535;                         // uint16 counters of refine_kernel
-                splits = (n_rows + rps - 1) / rps;
-                if (splits > 65535) return fail(IQW_ERR_UNSUPPORTED, "too many rows for the split grid");
-                g.grid = dim3((unsigned)slots, (unsigned)splits);
-                g.rows_per_split = rps;
-            }
+            if (int rc = plan_grid(n_rows, col_tiles, 4, 32, sms, &g)) return rc;
             // what select left open (nothing, as a rule) and the result rows: one cooperative launch
-            TailArgs ta{p, n_rows, n_cols, full, g.grid.x, g.grid.y, g.rows_per_split, rp, st, to_dB, eps, w, out};
+            TailArgs ta{p, n_rows, n_cols, g.grid.x, g.grid.y, g.rows_per_split, rp, st, to_dB, eps, w, out};
             int rc_tail = IQW_OK;
             { IQW_PROFILE("stats_tail", s);
-              IQW_DISPATCH_M(rp.n_ranks, rc_tail = launch_tail<M>(s, ta, sms)); }
+              rc_tail = dispatch_m<1>(rp.n_ranks, [&](auto M) { return launch_tail<M>(s, ta, sms); }); }
             if (rc_tail == IQW_ERR_UNSUPPORTED) {
-                // no cooperative launch on this device: the same steps as a train of kernels
-                // (7 x (refine, scan) + collect + resolve, then finalize; they exit at once when nothing is open)
+                // no cooperative launch on this device: the same steps as a train of kernels, then finalize
                 IQW_PROFILE_TRAIN("stats_tail_train", s, 2 * kRefineLevels + 3);
-                IQW_DISPATCH_M(rp.n_ranks, launch_refine_levels<M>(g, s, p, n_cols, full, rp, w, cblocks, cthreads, "stats"));
-                IQW_DISPATCH_M(rp.n_ranks, launch_collect<M>(g, s, p, n_cols, full, w, "stats_collect"));
-                { IQW_PROFILE_FINE("stats_resolve", s);
-                  resolve_kernel<<<(unsigned)n_cols, kResolveThreads, 0, s>>>(n_cols, rp, w); }
+                if (int rc = dispatch_m<1>(rp.n_ranks, [&](auto M) {
+                        return launch_interval_train<M>(g, s, p, n_rows, n_cols, rp, w, cblocks, cthreads);
+                    }))
+                    return rc;
                 { IQW_PROFILE_FINE("stats_finalize", s);
                   finalize_kernel<<<cblocks, cthreads, 0, s>>>(n_rows, n_cols, st, to_dB, eps, w, out); }
             } else if (rc_tail != IQW_OK) {
