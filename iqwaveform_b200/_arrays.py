@@ -73,11 +73,15 @@ def as_channels(x: torch.Tensor, axis: int) -> tuple[torch.Tensor, tuple, tuple]
         if t is not None:
             return t, lead, trail
         x = x.movedim(axis, -1)
-    n = x.shape[-1]
-    x2 = x.reshape(-1, n)
-    if x2.stride(-1) != 1 or (x2.shape[0] > 1 and x2.stride(0) < n):
-        x2 = x2.contiguous()
-    return x2, lead, trail
+    return unit_stride_rows(x.reshape(-1, x.shape[-1])), lead, trail
+
+
+def unit_stride_rows(x2: torch.Tensor) -> torch.Tensor:
+    """(C, N) rows of unit stride that do not overlap, as the kernels read them: `x2` itself when it is so laid
+    out (any row pitch >= N), else a contiguous copy"""
+    if x2.stride(-1) != 1 or (x2.shape[0] > 1 and x2.stride(0) < x2.shape[-1]):
+        return x2.contiguous()
+    return x2
 
 
 def _transpose_time_last(x: torch.Tensor, axis: int, lead: tuple, trail: tuple):

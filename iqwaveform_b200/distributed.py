@@ -22,14 +22,19 @@ The path shards without any collective on the data path, with one exception (the
   real exchange step of the path -- per-bin digit counts of a radix select are all_reduced
   (`select_order_statistics`; kernels in csrc/iqw_rowsplit.cu)
 
+Every time-axis planner returns a record of one layout: (first item the rank owns, one past its last, first
+item of the input it reads, one past the last it reads -- halo included --, items of the whole capture).  The
+owned items are frames, bins or outputs; the input is samples, or frames for `pfb_synth_shard`.  The field
+names say which; `_time_sharded` reads the records by position.
+
 Only the small results are exchanged: `gather_rows` is one `all_gather` over NCCL (CUDA tensors)
-or gloo (CPU tensors, used by the CPU tests) of the per-rank result rows.
+or gloo (CPU tensors, used by the CPU tests) of the per-rank result rows, or an exchange between the
+threads of a `ThreadGroup`.
 """
 from __future__ import annotations
 
 from typing import Callable, NamedTuple
 
-import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -97,14 +102,14 @@ def bin_shard(n_samples: int, bin_len: int, world: int, rank: int) -> BinShard:
 def gather_rows(local: torch.Tensor, sizes: list[int] | None = None, axis: int = 0, group=None) -> torch.Tensor:
     """all_gather of per-rank result rows along `axis`.  `sizes[r]` = rows of rank r when shards are
     ragged (default: every rank has local.shape[axis] rows).  Works on the backend of the group:
-    NCCL for CUDA tensors, gloo for CPU tensors."""
-    if not dist.is_initialized() or dist.get_world_size(group) == 1:
+    NCCL for CUDA tensors, gloo for CPU tensors; or between the threads of a `ThreadGroup`."""
+    world, rank = _world(group)
+    if world == 1:
         return local
-    world = dist.get_world_size(group)
     local = local.movedim(axis, 0).contiguous()
     if sizes is None:
         sizes = [local.shape[0]] * world
-    if len(sizes) != world or sizes[dist.get_rank(group)] != local.shape[0]:
+    if len(sizes) != world or sizes[rank] != local.shape[0]:
         raise ValueError('sizes must list the row count of every rank')
     rest = tuple(local.shape[1:])
     # equal-sized exchange (padded to the largest shard): one collective, KB-MB payloads
@@ -113,8 +118,11 @@ def gather_rows(local: torch.Tensor, sizes: list[int] | None = None, axis: int =
     if local.shape[0] < m:
         send = torch.zeros((m,) + rest, dtype=local.dtype, device=local.device)
         send[:local.shape[0]] = local
-    recv = [torch.empty((m,) + rest, dtype=local.dtype, device=local.device) for _ in range(world)]
-    dist.all_gather(recv, send, group=group)
+    if hasattr(group, 'iqw_all_reduce'):
+        recv = group.iqw_all_gather(send)
+    else:
+        recv = [torch.empty((m,) + rest, dtype=local.dtype, device=local.device) for _ in range(world)]
+        dist.all_gather(recv, send, group=group)
     out = torch.cat([r[:n] for r, n in zip(recv, sizes)], dim=0)
     return out.movedim(0, axis)
 
@@ -170,7 +178,8 @@ def _all_reduce(t: torch.Tensor, op: str, group=None) -> None:
 class ThreadGroup:
     """`ThreadGroup(n).member(r)` objects act as the `group` of rank r of n for the time-sharded
     functions when the n ranks are threads of ONE process (all shards on one GPU, or a CPU test):
-    all_reduce is a barrier plus an elementwise reduction over the members' tensors."""
+    all_reduce is a barrier plus an elementwise reduction over the members' tensors, all_gather a
+    barrier plus a copy of each."""
 
     def __init__(self, n: int):
         import threading
@@ -192,19 +201,30 @@ class _ThreadMember:
     def size(self) -> int:
         return self._o.n
 
-    def iqw_all_reduce(self, t: torch.Tensor, op: str) -> None:
+    def _exchange(self, t: torch.Tensor, combine: Callable):
+        """combine(the members' tensors in rank order), once every member has posted its `t`; no member
+        returns before all have combined"""
         o = self._o
         o._slots[self._r] = t
         o._barrier.wait()
-        stacked = torch.stack(list(o._slots))
-        res = {'sum': stacked.sum(0), 'min': stacked.amin(0), 'max': stacked.amax(0)}[op].to(t.dtype)
+        res = combine(list(o._slots))
         if t.is_cuda:
             torch.cuda.synchronize()
         o._barrier.wait()
-        t.copy_(res)
+        return res
+
+    def iqw_all_reduce(self, t: torch.Tensor, op: str) -> None:
+        def reduce(ts):
+            stacked = torch.stack(ts)
+            return {'sum': stacked.sum(0), 'min': stacked.amin(0), 'max': stacked.amax(0)}[op].to(t.dtype)
+        t.copy_(self._exchange(t, reduce))
         if t.is_cuda:
             torch.cuda.synchronize()
-        o._barrier.wait()
+        self._o._barrier.wait()
+
+    def iqw_all_gather(self, t: torch.Tensor) -> list[torch.Tensor]:
+        # copies: a member may change its tensor as soon as the exchange is over
+        return self._exchange(t, lambda ts: [s.clone() for s in ts])
 
 
 def persistence_spectrum_sharded(x_local, *, n_channels: int, group=None, compute: Callable | None = None, **kw):
@@ -492,53 +512,74 @@ def persistence_spectrum_time_sharded(x_halo, *, n_samples: int, fs: float, wind
     return out
 
 
+def _time_sharded(x_halo, plan: Callable, run: Callable, compute: Callable | None, default: Callable, *, group,
+                  gather: bool, ndim: int | None = 1, unit: str = 'samples'):
+    """the steps every time-sharded entry point shares.  `plan(world, rank)` returns a shard record (the layout
+    of the module docstring) whose read span `x_halo` holds: along its first axis and with `ndim` axes, or along
+    its last axis when ndim is None.  Returns `run(compute, shard)` (`compute` defaulting to `default`) as a
+    tensor or, with `gather`, the owned items of all ranks on every rank."""
+    world, rank = _world(group)
+    sh = plan(world, rank)
+    own0, own1, read0, read1, _ = sh
+    n = read1 - read0
+    if ndim is None:
+        bad, want = x_halo.shape[-1] != n, f'{n} {unit}'
+    else:
+        bad = x_halo.ndim != ndim or x_halo.shape[0] != n
+        want = f'a {"1-D " if ndim == 1 else ""}shard of {n} {unit}'
+    if bad:
+        raise ValueError(f'rank {rank} expects {want}, got {tuple(x_halo.shape)}')
+    y = torch.as_tensor(run(default if compute is None else compute, sh))
+    assert y.shape[0] == own1 - own0
+    if not gather:
+        return y
+    return gather_rows(y, [s[1] - s[0] for s in (plan(world, r) for r in range(world))], 0, group)
+
+
+def _on_device(device_op: Callable, not_built: str) -> Callable:
+    """`device_op` of (C, ...) complex64 rows on the device as the `compute` of a rank's shard: the shard goes to
+    the device as one row.  `not_built` is the NotImplementedError message for a shard of another dtype."""
+    def compute(x, *args, **kw):
+        from . import _arrays
+        xd, _ = _arrays.to_device(x)
+        if xd.dtype != torch.complex64:
+            raise NotImplementedError(f'{not_built} (got {xd.dtype})')
+        return device_op(xd[None], *args, **kw)[0]
+    return compute
+
+
 def spectrogram_time_sharded(x_halo, *, n_samples: int, nperseg: int, noverlap: int = 0, group=None,
                              compute: Callable | None = None, gather: bool = False, **kw):
     """time-sharded spectrogram of a 1-D capture of `n_samples` samples: `x_halo` holds this rank's
     samples [shard.sample0, shard.sample1) (halo included).  Returns this rank's frames
     (T_local, nfft) or, with gather=True, all frames on every rank."""
-    if compute is None:
-        from .fourier import spectrogram as compute
-    world, rank = _world(group)
-    sh = frame_shard(n_samples, nperseg, noverlap, world, rank)
-    if x_halo.shape[-1] != sh.sample1 - sh.sample0:
-        raise ValueError(f'rank {rank} expects {sh.sample1 - sh.sample0} samples, got {x_halo.shape[-1]}')
-    p = compute(x_halo, nperseg=nperseg, noverlap=noverlap, axis=0, return_axis_arrays=False, **kw)
-    p = torch.as_tensor(p)
-    assert p.shape[0] == sh.frame1 - sh.frame0
-    if not gather or world == 1:
-        return p
-    sizes = [(lambda s: s.frame1 - s.frame0)(frame_shard(n_samples, nperseg, noverlap, world, r)) for r in range(world)]
-    return gather_rows(p, sizes, 0, group)
+    from . import fourier
+    return _time_sharded(x_halo, lambda w, r: frame_shard(n_samples, nperseg, noverlap, w, r),
+                         lambda f, sh: f(x_halo, nperseg=nperseg, noverlap=noverlap, axis=0, return_axis_arrays=False,
+                                         **kw),
+                         compute, fourier.spectrogram, group=group, gather=gather, ndim=None)
 
 
 def iq_to_bin_power_sharded(x_local, Ts: float, Tbin: float, *, n_samples: int, kind='mean', group=None,
                             compute: Callable | None = None):
     """bin-sharded iq_to_bin_power of a 1-D capture: `x_local` holds samples
     [shard.sample0, shard.sample1); every rank returns all n_bins values."""
-    if compute is None:
-        from .power_analysis import iq_to_bin_power as compute
-    world, rank = _world(group)
+    from . import power_analysis
     bin_len = round(Tbin / Ts)
-    sh = bin_shard(n_samples, bin_len, world, rank)
-    if x_local.shape[-1] != sh.sample1 - sh.sample0:
-        raise ValueError(f'rank {rank} expects {sh.sample1 - sh.sample0} samples, got {x_local.shape[-1]}')
-    out = torch.as_tensor(compute(x_local, Ts, Tbin, kind=kind, axis=0, truncate=True))
-    if world == 1:
-        return out
-    sizes = [(lambda s: s.bin1 - s.bin0)(bin_shard(n_samples, bin_len, world, r)) for r in range(world)]
-    return gather_rows(out, sizes, 0, group)
+    return _time_sharded(x_local, lambda w, r: bin_shard(n_samples, bin_len, w, r),
+                         lambda f, sh: f(x_local, Ts, Tbin, kind=kind, axis=0, truncate=True),
+                         compute, power_analysis.iq_to_bin_power, group=group, gather=True, ndim=None)
 
 
-class UpfirdnShard(NamedTuple):
-    out0: int       # first output of this rank
+class OutputShard(NamedTuple):
+    out0: int       # first output of this rank (for oaconvolve: an index into the output of the chosen mode)
     out1: int       # one past its last output
     sample0: int    # first sample it reads
     sample1: int    # one past the last sample it reads (includes the halo)
     n_out: int      # outputs of the whole capture
 
 
-def upfirdn_shard(n_in: int, n_taps: int, up: int, down: int, world: int, rank: int) -> UpfirdnShard:
+def upfirdn_shard(n_in: int, n_taps: int, up: int, down: int, world: int, rank: int) -> OutputShard:
     """time-axis shard of upfirdn: outputs split evenly; the samples are those the rank's outputs read,
     y[n] = sum_{j < Lp} hp[p][j] * x[n*down div up - j], clamped to [0, n_in)"""
     from . import _plan
@@ -549,10 +590,10 @@ def upfirdn_shard(n_in: int, n_taps: int, up: int, down: int, world: int, rank: 
     lp = -(-n_taps // up)
     if o1 == o0:
         s = min(o0 * down // up, n_in)
-        return UpfirdnShard(o0, o1, s, s, n_out)
+        return OutputShard(o0, o1, s, s, n_out)
     s0 = max(0, o0 * down // up - (lp - 1))
     s1 = min(n_in, (o1 - 1) * down // up + 1)
-    return UpfirdnShard(o0, o1, s0, max(s0, s1), n_out)
+    return OutputShard(o0, o1, s0, max(s0, s1), n_out)
 
 
 def upfirdn_time_sharded(x_halo, h, up: int = 1, down: int = 1, *, n_samples: int, group=None,
@@ -565,35 +606,14 @@ def upfirdn_time_sharded(x_halo, h, up: int = 1, down: int = 1, *, n_samples: in
     from . import fourier
     up, down = int(up), int(down)
     table, n_taps = fourier._upfirdn_taps(h, up, down)
-    world, rank = _world(group)
-    sh = upfirdn_shard(n_samples, n_taps, up, down, world, rank)
-    if x_halo.ndim != 1 or x_halo.shape[0] != sh.sample1 - sh.sample0:
-        raise ValueError(f'rank {rank} expects a 1-D shard of {sh.sample1 - sh.sample0} samples, got {tuple(x_halo.shape)}')
-    if compute is None:
-        from . import _arrays
-        xd, _ = _arrays.to_device(x_halo)
-        if xd.dtype != torch.complex64:
-            raise NotImplementedError(f'upfirdn: only complex64 x is built (got {xd.dtype})')
-        y = fourier._upfirdn_device(xd.reshape(1, -1), table, n_taps, up, down, x_first=sh.sample0,
-                                    out_first=sh.out0, n_out=sh.out1 - sh.out0)[0]
-    else:
-        y = torch.as_tensor(compute(x_halo, table, n_taps, up, down, x_first=sh.sample0, out_first=sh.out0,
-                                    n_out=sh.out1 - sh.out0))
-    if not gather or world == 1:
-        return y
-    sizes = [(lambda s: s.out1 - s.out0)(upfirdn_shard(n_samples, n_taps, up, down, world, r)) for r in range(world)]
-    return gather_rows(y, sizes, 0, group)
+    return _time_sharded(x_halo, lambda w, r: upfirdn_shard(n_samples, n_taps, up, down, w, r),
+                         lambda f, sh: f(x_halo, table, n_taps, up, down, x_first=sh.sample0, out_first=sh.out0,
+                                         n_out=sh.out1 - sh.out0),
+                         compute, _on_device(fourier._upfirdn_device, 'upfirdn: only complex64 x is built'),
+                         group=group, gather=gather)
 
 
-class OaconvolveShard(NamedTuple):
-    out0: int       # first output of this rank (index into the output of the chosen mode)
-    out1: int       # one past its last output
-    sample0: int    # first sample it reads
-    sample1: int    # one past the last sample it reads (includes the halo)
-    n_out: int      # outputs of the whole capture in the chosen mode
-
-
-def oaconvolve_shard(n_in: int, n_taps: int, mode: str, world: int, rank: int) -> OaconvolveShard:
+def oaconvolve_shard(n_in: int, n_taps: int, mode: str, world: int, rank: int) -> OutputShard:
     """time-axis shard of oaconvolve(x, h, mode) for a capture of n_in samples and an n_taps filter:
     the outputs of the mode are split evenly; the samples are every in-range sample of the overlap-save
     blocks those outputs fall in (block b reads [b*hop - D, b*hop - D + nfft)), clamped to [0, n_in).
@@ -608,11 +628,11 @@ def oaconvolve_shard(n_in: int, n_taps: int, mode: str, world: int, rank: int) -
     o0, o1 = _split(n_out, world, rank)
     if o1 == o0:
         s = min(max(0, (first + o0) // hop * hop - discard), n_in)
-        return OaconvolveShard(o0, o1, s, s, n_out)
+        return OutputShard(o0, o1, s, s, n_out)
     b0, b1 = (first + o0) // hop, (first + o1 - 1) // hop
     s0 = min(n_in, max(0, b0 * hop - discard))
     s1 = min(n_in, b1 * hop - discard + nfft)
-    return OaconvolveShard(o0, o1, s0, max(s0, s1), n_out)
+    return OutputShard(o0, o1, s0, max(s0, s1), n_out)
 
 
 def oaconvolve_time_sharded(x_halo, h, mode: str = 'full', *, n_samples: int, group=None,
@@ -624,42 +644,20 @@ def oaconvolve_time_sharded(x_halo, h, mode: str = 'full', *, n_samples: int, gr
     `compute(x_halo, hspec, n_taps, nfft, discard, x_first=, out_first=, n_out=)` defaults to the CUDA
     kernel."""
     from . import _plan, fourier
-    if isinstance(h, torch.Tensor):
-        h = h.detach().cpu().numpy()
-    h = np.asarray(h)
-    if h.ndim != 1 or h.size == 0:
+    h = fourier._as_operand(h)
+    if h.ndim != 1 or h.shape[0] == 0:
         raise ValueError('oaconvolve_time_sharded: h must be 1-D with non-zero length')
-    world, rank = _world(group)
-    sh = oaconvolve_shard(n_samples, h.size, mode, world, rank)
-    if x_halo.ndim != 1 or x_halo.shape[0] != sh.sample1 - sh.sample0:
-        raise ValueError(f'rank {rank} expects a 1-D shard of {sh.sample1 - sh.sample0} samples, got {tuple(x_halo.shape)}')
-    nfft, discard = _plan.oaconvolve_plan(h.size)
-    hspec = _plan.oaconvolve_spectrum(h[None], nfft)
-    first, _ = _plan.oaconvolve_window(mode, n_samples, h.size)
-    kw = dict(x_first=sh.sample0, out_first=first + sh.out0, n_out=sh.out1 - sh.out0)
-    if compute is None:
-        from . import _arrays
-        xd, _ = _arrays.to_device(x_halo)
-        if xd.dtype != torch.complex64:
-            raise NotImplementedError(f'oaconvolve: only a complex64 signal is built (got {xd.dtype})')
-        y = fourier._oaconvolve_device(xd.reshape(1, -1), hspec, h.size, nfft, discard, **kw)[0]
-    else:
-        y = torch.as_tensor(compute(x_halo, hspec, h.size, nfft, discard, **kw))
-    if not gather or world == 1:
-        return y
-    sizes = [(lambda s: s.out1 - s.out0)(oaconvolve_shard(n_samples, h.size, mode, world, r)) for r in range(world)]
-    return gather_rows(y, sizes, 0, group)
+    hspec, n_taps, nfft, discard = fourier._oaconvolve_filter(h, 0)
+    first, _ = _plan.oaconvolve_window(mode, n_samples, n_taps)
+    return _time_sharded(x_halo, lambda w, r: oaconvolve_shard(n_samples, n_taps, mode, w, r),
+                         lambda f, sh: f(x_halo, hspec, n_taps, nfft, discard, x_first=sh.sample0,
+                                         out_first=first + sh.out0, n_out=sh.out1 - sh.out0),
+                         compute, _on_device(fourier._oaconvolve_device,
+                                             'oaconvolve: only a complex64 signal is built'),
+                         group=group, gather=gather)
 
 
-class PfbShard(NamedTuple):
-    frame0: int     # first frame of this rank
-    frame1: int     # one past its last frame
-    sample0: int    # first sample it reads
-    sample1: int    # one past the last sample it reads (includes the halo)
-    n_frames: int   # frames of the whole capture
-
-
-def pfb_shard(n_samples: int, n_taps: int, nchannels: int, hop: int | None, world: int, rank: int) -> PfbShard:
+def pfb_shard(n_samples: int, n_taps: int, nchannels: int, hop: int | None, world: int, rank: int) -> FrameShard:
     """time-axis shard of pfb_channelize(x, h, nchannels, hop) for a capture of n_samples samples and an n_taps
     prototype: the frames are split evenly, and rank r reads the samples [frame0*hop, (frame1 - 1)*hop + L) of
     its frames -- a halo of L - hop samples past the frame0*hop of the next rank.  A frame's bits depend only
@@ -672,8 +670,8 @@ def pfb_shard(n_samples: int, n_taps: int, nchannels: int, hop: int | None, worl
     f0, f1 = _split(T, world, rank)
     if f1 == f0:
         s = min(f0 * hop, n_samples)
-        return PfbShard(f0, f1, s, s, T)
-    return PfbShard(f0, f1, f0 * hop, (f1 - 1) * hop + n_taps, T)
+        return FrameShard(f0, f1, s, s, T)
+    return FrameShard(f0, f1, f0 * hop, (f1 - 1) * hop + n_taps, T)
 
 
 def pfb_channelize_time_sharded(x_halo, h, nchannels, hop=None, *, n_samples: int, group=None,
@@ -686,23 +684,11 @@ def pfb_channelize_time_sharded(x_halo, h, nchannels, hop=None, *, n_samples: in
     kernel."""
     from . import fourier
     taps, L, K, hop = fourier._pfb_args(h, nchannels, hop)
-    world, rank = _world(group)
-    sh = pfb_shard(n_samples, L, K, hop, world, rank)
-    if x_halo.ndim != 1 or x_halo.shape[0] != sh.sample1 - sh.sample0:
-        raise ValueError(f'rank {rank} expects a 1-D shard of {sh.sample1 - sh.sample0} samples, got {tuple(x_halo.shape)}')
-    kw = dict(x_first=sh.sample0, frame_first=sh.frame0, n_frames=sh.frame1 - sh.frame0)
-    if compute is None:
-        from . import _arrays
-        xd, _ = _arrays.to_device(x_halo)
-        if xd.dtype != torch.complex64:
-            raise NotImplementedError(f'pfb_channelize: only a complex64 signal is built (got {xd.dtype})')
-        y = fourier._pfb_device(xd.reshape(1, -1), taps, L, K, hop, **kw)[0]
-    else:
-        y = torch.as_tensor(compute(x_halo, taps, L, K, hop, **kw))
-    if not gather or world == 1:
-        return y
-    sizes = [(lambda s: s.frame1 - s.frame0)(pfb_shard(n_samples, L, K, hop, world, r)) for r in range(world)]
-    return gather_rows(y, sizes, 0, group)
+    return _time_sharded(x_halo, lambda w, r: pfb_shard(n_samples, L, K, hop, w, r),
+                         lambda f, sh: f(x_halo, taps, L, K, hop, x_first=sh.sample0, frame_first=sh.frame0,
+                                         n_frames=sh.frame1 - sh.frame0),
+                         compute, _on_device(fourier._pfb_device, 'pfb_channelize: only a complex64 signal is built'),
+                         group=group, gather=gather)
 
 
 class PfbSynthShard(NamedTuple):
@@ -745,20 +731,9 @@ def pfb_synthesize_time_sharded(y_halo, g, hop=None, *, n_frames: int, group=Non
     if y_halo.ndim != 2:
         raise ValueError(f'pfb_synthesize_time_sharded: y_halo must be (frames, nchannels), got {tuple(y_halo.shape)}')
     taps, Lg, K, hop = fourier._pfb_args(g, y_halo.shape[1], hop, what='pfb_synthesize', name='g')
-    world, rank = _world(group)
-    sh = pfb_synth_shard(n_frames, Lg, K, hop, world, rank)
-    if y_halo.shape[0] != sh.frame1 - sh.frame0:
-        raise ValueError(f'rank {rank} expects a shard of {sh.frame1 - sh.frame0} frames, got {tuple(y_halo.shape)}')
-    kw = dict(frame_first=sh.frame0, n_frames_total=n_frames, out_first=sh.out0, n_out=sh.out1 - sh.out0)
-    if compute is None:
-        from . import _arrays
-        yd, _ = _arrays.to_device(y_halo)
-        if yd.dtype != torch.complex64:
-            raise NotImplementedError(f'pfb_synthesize: only complex64 frames are built (got {yd.dtype})')
-        x = fourier._pfb_synth_device(yd.reshape(1, -1, K), taps, Lg, hop, **kw)[0]
-    else:
-        x = torch.as_tensor(compute(y_halo, taps, Lg, hop, **kw))
-    if not gather or world == 1:
-        return x
-    sizes = [(lambda s: s.out1 - s.out0)(pfb_synth_shard(n_frames, Lg, K, hop, world, r)) for r in range(world)]
-    return gather_rows(x, sizes, 0, group)
+    return _time_sharded(y_halo, lambda w, r: pfb_synth_shard(n_frames, Lg, K, hop, w, r),
+                         lambda f, sh: f(y_halo, taps, Lg, hop, frame_first=sh.frame0, n_frames_total=n_frames,
+                                         out_first=sh.out0, n_out=sh.out1 - sh.out0),
+                         compute, _on_device(fourier._pfb_synth_device,
+                                             'pfb_synthesize: only complex64 frames are built'),
+                         group=group, gather=gather, ndim=2, unit='frames')

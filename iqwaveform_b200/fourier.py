@@ -557,9 +557,8 @@ def _upfirdn_device(x2: torch.Tensor, table: np.ndarray, n_taps: int, up: int, d
     """(C, N) complex64 device rows holding global samples [x_first, x_first + N) -> (C, n_out) outputs
     [out_first, out_first + n_out) of the whole capture.  The kernel reads unit-stride rows: any other
     layout (a column of an (N, C) capture, a strided view) is copied first."""
+    x2 = _arrays.unit_stride_rows(x2)
     C, N = x2.shape
-    if x2.stride(1) != 1 or (C > 1 and x2.stride(0) < N):
-        x2 = x2.contiguous()
     y = torch.empty((C, n_out), dtype=torch.complex64, device=x2.device)
     if n_out == 0 or C == 0:
         return y
@@ -651,14 +650,25 @@ def _oaconvolve_roles(s1: tuple, s2: tuple, mode: str, axes):
     return a, signal_is_in1, per_row
 
 
+def _oaconvolve_filter(h, a: int) -> tuple[np.ndarray, int, int, int]:
+    """(spectrum rows, n_taps, nfft, discard) of the filter `h` (numpy, or torch on the host or the device) along
+    its axis `a`: one spectrum row per filter row.  NotImplementedError for a filter that is not numeric."""
+    if isinstance(h, torch.Tensor):
+        h = h.detach().cpu().numpy()
+    if not (np.issubdtype(h.dtype, np.number) or h.dtype == np.bool_):
+        raise NotImplementedError(f'oaconvolve: a filter of dtype {h.dtype} is not built')
+    n_taps = h.shape[a]
+    nfft, discard = _plan.oaconvolve_plan(n_taps)
+    return _plan.oaconvolve_spectrum(np.moveaxis(h, a, -1).reshape(-1, n_taps), nfft), n_taps, nfft, discard
+
+
 def _oaconvolve_device(x2: torch.Tensor, hspec: np.ndarray, n_taps: int, nfft: int, discard: int, *,
                        x_first: int = 0, out_first: int, n_out: int) -> torch.Tensor:
     """(C, N) complex64 device rows holding global samples [x_first, x_first + N) -> (C, n_out) outputs
     [out_first, out_first + n_out) of the full convolution.  `hspec`: (1 | C, nfft) complex64 spectrum rows
     (_plan.oaconvolve_spectrum).  The kernel reads unit-stride rows: any other layout is copied first."""
+    x2 = _arrays.unit_stride_rows(x2)
     C, N = x2.shape
-    if x2.stride(1) != 1 or (C > 1 and x2.stride(0) < N):
-        x2 = x2.contiguous()
     y = torch.empty((C, n_out), dtype=torch.complex64, device=x2.device)
     if n_out == 0 or C == 0:
         return y
@@ -705,14 +715,8 @@ def oaconvolve(in1, in2, mode='full', axes=None):
     x, h = (in1, in2) if signal_is_in1 else (in2, in1)
     if x.dtype not in (np.complex64, torch.complex64):
         raise NotImplementedError(f'oaconvolve: only a complex64 signal is built (got {x.dtype})')
-    if isinstance(h, torch.Tensor):
-        h = h.detach().cpu().numpy()
-    if not (np.issubdtype(h.dtype, np.number) or h.dtype == np.bool_):
-        raise NotImplementedError(f'oaconvolve: a filter of dtype {h.dtype} is not built')
-    n_taps = h.shape[a]
+    hspec, n_taps, nfft, discard = _oaconvolve_filter(h, a)
     first, n_out = _plan.oaconvolve_window(mode, s1[a], s2[a])
-    nfft, discard = _plan.oaconvolve_plan(n_taps)
-    hspec = _plan.oaconvolve_spectrum(np.moveaxis(h, a, -1).reshape(-1, n_taps), nfft)
     xd, res = _arrays.to_device(x)
     if mode == 'same' and not signal_is_in1:
         # scipy centres 'same' on in1's shape on every axis: where the (broadcast) filter in1 has size 1, the
@@ -758,9 +762,8 @@ def _pfb_device(x2: torch.Tensor, taps: np.ndarray, n_taps: int, nfft: int, hop:
     """(C, N) complex64 device rows holding global samples [x_first, x_first + N) -> (C, n_frames, nfft),
     frames [frame_first, frame_first + n_frames).  The kernel reads unit-stride rows: any other layout is
     copied first."""
+    x2 = _arrays.unit_stride_rows(x2)
     C, N = x2.shape
-    if x2.stride(1) != 1 or (C > 1 and x2.stride(0) < N):
-        x2 = x2.contiguous()
     y = torch.empty((C, n_frames, nfft), dtype=torch.complex64, device=x2.device)
     if n_frames == 0 or C == 0:
         return y

@@ -4,7 +4,6 @@ scipy.signal.convolve in float64 within the documented bound, and run shard by s
 planner's spans, bitwise equal to one call."""
 import numpy as np
 import pytest
-import scipy.fft as sf
 import scipy.signal as ss
 import torch
 
@@ -12,33 +11,11 @@ import iqwaveform_b200 as iqw
 from iqwaveform_b200 import _plan
 from iqwaveform_b200 import distributed as D
 
+from _oaconvolve_numpy import emulate
+
 # the (nfft, nfft/discard) pairs csrc/iqw_oaconvolve.cu instantiates (oaconvolve_built)
 BUILT = {(16, 4), (16, 8), (16, 16), (32, 4), (64, 4), (256, 8), (512, 8), (1024, 8), (2048, 8), (4096, 8),
          (8192, 2), (8192, 4), (8192, 8)}
-
-
-def _emulate(x_buf, hspec, n_taps, nfft, discard, *, x_first, out_first, n_out):
-    """the kernel's blocks in numpy complex64: block b reads global samples [b*hop - D, b*hop - D + nfft)
-    of the buffer that holds [x_first, x_first + len(x_buf)) (zero elsewhere), forward FFT, times H,
-    inverse as conj(FFT(conj(.))), keeps samples D.. as outputs [b*hop, b*hop + hop).  One block at a time,
-    so that a block's bits cannot depend on what else is transformed with it."""
-    x_buf = np.asarray(x_buf)
-    H = hspec[0]
-    hop = nfft - discard
-    y = np.zeros(n_out, np.complex64)
-    if n_out == 0:
-        return y
-    for b in range(out_first // hop, (out_first + n_out - 1) // hop + 1):
-        g0 = b * hop - discard - x_first
-        blk = np.zeros(nfft, np.complex64)
-        lo, hi = max(g0, 0), min(g0 + nfft, x_buf.size)
-        if hi > lo:
-            blk[lo - g0:hi - g0] = x_buf[lo:hi]
-        kept = np.conj(sf.fft(np.conj(sf.fft(blk, workers=1) * H), workers=1))[discard:]
-        n0 = b * hop - out_first
-        a0, a1 = max(n0, 0), min(n0 + hop, n_out)
-        y[a0:a1] = kept[a0 - n0:a1 - n0]
-    return y
 
 
 def _bound(x, h, mode, n1, n2, factor):
@@ -157,7 +134,7 @@ def test_emulation_within_bound_of_float64(M, cplx):
     hspec = _plan.oaconvolve_spectrum(h[None], nfft)
     for mode in ('full', 'same', 'valid'):
         first, n = _plan.oaconvolve_window(mode, N, M)
-        got = _emulate(x, hspec, M, nfft, discard, x_first=0, out_first=first, n_out=n)
+        got = emulate(x, hspec, M, nfft, discard, x_first=0, out_first=first, n_out=n)
         want = ss.convolve(x.astype(np.complex128), h, mode=mode)
         err = np.abs(got - want)
         # 3x: scipy's float32 FFT reaches 2.2 units on the 16-point blocks of a 2-tap filter, < 2 elsewhere
@@ -175,8 +152,8 @@ def test_shards_are_bitwise_one_call(world, mode):
         x = _signal(rng, N)
         nfft, discard = _plan.oaconvolve_plan(M)
         first, n = _plan.oaconvolve_window(mode, N, M)
-        single = _emulate(x, _plan.oaconvolve_spectrum(h[None], nfft), M, nfft, discard, x_first=0,
-                          out_first=first, n_out=n)
+        single = emulate(x, _plan.oaconvolve_spectrum(h[None], nfft), M, nfft, discard, x_first=0,
+                         out_first=first, n_out=n)
         group = D.ThreadGroup(world)
         outs, parts = [], []
         for r in range(world):
@@ -184,7 +161,7 @@ def test_shards_are_bitwise_one_call(world, mode):
             assert sh.n_out == n and 0 <= sh.sample0 <= sh.sample1 <= N
             outs += list(range(sh.out0, sh.out1))
             parts.append(np.asarray(D.oaconvolve_time_sharded(x[sh.sample0:sh.sample1], h, mode, n_samples=N,
-                                                              group=group.member(r), compute=_emulate)))
+                                                              group=group.member(r), compute=emulate)))
         assert outs == list(range(n))
         assert np.array_equal(np.concatenate(parts), single), (N, M)
 
@@ -201,6 +178,6 @@ def test_shard_rejects_a_wrong_halo_and_a_short_capture():
     sh = D.oaconvolve_shard(1000, 33, 'full', 2, 1)
     x = np.zeros(sh.sample1 - sh.sample0 + 1, np.complex64)
     with pytest.raises(ValueError, match='expects a 1-D shard'):
-        D.oaconvolve_time_sharded(x, np.ones(33), n_samples=1000, group=D.ThreadGroup(2).member(1), compute=_emulate)
+        D.oaconvolve_time_sharded(x, np.ones(33), n_samples=1000, group=D.ThreadGroup(2).member(1), compute=emulate)
     with pytest.raises(NotImplementedError):
         D.oaconvolve_shard(10, 33, 'full', 2, 0)

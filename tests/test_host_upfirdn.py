@@ -11,19 +11,7 @@ import iqwaveform_b200 as iqw
 from iqwaveform_b200 import _plan
 from iqwaveform_b200 import distributed as D
 
-
-def _direct(x_buf, table, n_taps, up, down, *, x_first, out_first, n_out):
-    """float64 y[n] = sum_j hp[p][j] * x[i0 - j] over global outputs [out_first, out_first + n_out), reading
-    only the buffer that holds global samples [x_first, x_first + len(x_buf)) (zero elsewhere)"""
-    x_buf = np.asarray(x_buf).astype(np.complex128)
-    rows, lp = table.shape
-    p, i0 = _plan.upfirdn_phase_index(np.arange(out_first, out_first + n_out), up, down)
-    y = np.zeros(n_out, np.complex128)
-    for j in range(lp):
-        idx = i0 - j - x_first
-        ok = (idx >= 0) & (idx < x_buf.size) & (p < rows)
-        y[ok] += table[p[ok], j].astype(np.complex128) * x_buf[idx[ok]]
-    return y
+from _upfirdn_numpy import direct
 
 
 GRID = [(L, n, up, down) for L in (1, 2, 7, 16, 161) for n in (1, 2, 5, 64, 999)
@@ -55,7 +43,7 @@ def test_direct_formula_is_scipy():
         x = (rng.standard_normal(n) + 1j * rng.standard_normal(n)).astype(np.complex64)
         want = ss.upfirdn(h.astype(np.float64), x.astype(np.complex128), up, down)
         t = _plan.upfirdn_polyphase(h, up)
-        got = _direct(x, t, L, up, down, x_first=0, out_first=0, n_out=want.size)
+        got = direct(x, t, L, up, down, x_first=0, out_first=0, n_out=want.size)
         np.testing.assert_allclose(got, want, rtol=1e-12, atol=1e-12)
 
 
@@ -75,7 +63,7 @@ def test_shard_planner_tiles_outputs_and_holds_every_input(world):
             assert 0 <= sh.sample0 <= sh.sample1 <= n
             outs += list(range(sh.out0, sh.out1))
             parts.append(np.asarray(D.upfirdn_time_sharded(x[sh.sample0:sh.sample1], h, up, down, n_samples=n,
-                                                           group=group.member(r), compute=_direct)))
+                                                           group=group.member(r), compute=direct)))
         assert outs == list(range(want.size))
         np.testing.assert_allclose(np.concatenate(parts), want, rtol=1e-10, atol=1e-10)
 
@@ -84,7 +72,7 @@ def test_shard_rejects_a_wrong_halo():
     sh = D.upfirdn_shard(1000, 33, 2, 3, 2, 1)
     x = np.zeros(sh.sample1 - sh.sample0 + 1, np.complex64)
     with pytest.raises(ValueError, match='expects a 1-D shard'):
-        D.upfirdn_time_sharded(x, np.ones(33), 2, 3, n_samples=1000, group=D.ThreadGroup(2).member(1), compute=_direct)
+        D.upfirdn_time_sharded(x, np.ones(33), 2, 3, n_samples=1000, group=D.ThreadGroup(2).member(1), compute=direct)
 
 
 def test_argument_errors_before_device_work():
