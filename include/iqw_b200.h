@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define IQW_ABI_VERSION 12
+#define IQW_ABI_VERSION 13
 
 typedef enum iqw_status {
     IQW_OK = 0,
@@ -366,6 +366,52 @@ int iqw_pfb_synthesize_c64(const void* d_y, int64_t n_channels, int64_t n_frames
                            int64_t frame_first, int64_t n_frames_total, const void* d_taps, int32_t n_taps,
                            int32_t nfft, int32_t hop, int64_t out_first, int64_t n_out, void* d_out,
                            int64_t out_channel_stride, void* d_workspace, size_t workspace_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Kernel 10 (csrc/iqw_sosfilt.cu): scipy.signal.sosfilt of complex64 rows by a cascade of S second-order
+ * sections in direct form II transposed, real float32 coefficients (no reference counterpart: the reference
+ * has no IIR filter).  Per section s and sample:  y = b0 u + z1,  z1 = b1 u - a1 y + z2,  z2 = b2 u - a2 y.
+ *
+ * The cascade is one linear system of 2S states (z1_0, z2_0, z1_1, ..., scipy's zi order), z[n+1] = A z[n] +
+ * B x[n].  A row is cut into chunks of L samples, G chunks to a group and H groups to a carry block, anchored at
+ * sample 0; iqw_sosfilt_geometry returns (L, G, H), which depend on S alone.  Three passes:
+ *   states  each chunk's final state from a zero state (fp32, to the workspace), and each group's zero-state
+ *           final state b_g, folded from them in float64 with A^L
+ *   carry   the start state s_g of every group: s_{g+1} = A^(LG) s_g + b_g from s_0 = zi, in float64, folded
+ *           in carry blocks of H groups with A^(LGH) between blocks
+ *   apply   each chunk's start state expanded from s_g in float64, rounded to complex64; the chunk is filtered
+ *           again from it and y written; zf is the state after the last sample
+ * iqw_sosfilt_c64 is exactly states + carry + apply, so a capture split into time shards on group boundaries,
+ * whose group states are concatenated before one carry, gives the bits of one call.
+ *
+ *   h_sos         HOST float32 (n_sections, 6): b0 b1 b2 a0 a1 a2 per section, a0 == 1 (else IQW_ERR_INVALID);
+ *                 1 <= n_sections <= 16 (else IQW_ERR_UNSUPPORTED)
+ *   d_powers      float64 (3, 2S, 2S) row-major: A^L, A^(L*G), A^(L*G*H) for the A of the float32 sos
+ *                 (python: iqwaveform_b200._plan.sosfilt_powers)
+ *   d_x / d_y     (n_rows, n_samples) complex64, row strides in elements; n_rows <= 65535
+ *   d_group_states complex128 (n_rows, n_groups, 2S), n_groups = ceil(n_samples / (L*G)): b_g written by
+ *                 states, turned into s_g in place by carry, read by apply; 16-byte aligned
+ *   d_zi / d_zf   complex64 (n_rows, 2S) start / final states, or null (zero start; no final state)
+ *   d_workspace   states / apply: the chunk states, >= iqw_sosfilt_workspace_bytes(n_rows, n_samples, S);
+ *                 carry: >= iqw_sosfilt_carry_workspace_bytes(n_rows, n_groups, S); iqw_sosfilt_c64: >=
+ *                 iqw_sosfilt_workspace_bytes, holding the group states too.  16-byte aligned.
+ * The queries need no GPU and return 0 for bad arguments. */
+int iqw_sosfilt_geometry(int32_t n_sections, int32_t* out3);
+size_t iqw_sosfilt_workspace_bytes(int64_t n_rows, int64_t n_samples, int32_t n_sections);
+size_t iqw_sosfilt_carry_workspace_bytes(int64_t n_rows, int64_t n_groups, int32_t n_sections);
+int iqw_sosfilt_states_c64(const void* d_x, int64_t n_rows, int64_t n_samples, int64_t x_row_stride,
+                           const float* h_sos, int32_t n_sections, const void* d_powers, void* d_group_states,
+                           void* d_workspace, size_t workspace_bytes, void* stream);
+int iqw_sosfilt_carry_c64(void* d_group_states, int64_t n_rows, int64_t n_groups, const void* d_zi,
+                          int32_t n_sections, const void* d_powers, void* d_workspace, size_t workspace_bytes,
+                          void* stream);
+int iqw_sosfilt_apply_c64(const void* d_x, int64_t n_rows, int64_t n_samples, int64_t x_row_stride,
+                          const float* h_sos, int32_t n_sections, const void* d_powers, const void* d_group_states,
+                          const void* d_workspace, size_t workspace_bytes, void* d_y, int64_t y_row_stride,
+                          void* d_zf, void* stream);
+int iqw_sosfilt_c64(const void* d_x, int64_t n_rows, int64_t n_samples, int64_t x_row_stride, const float* h_sos,
+                    int32_t n_sections, const void* d_powers, const void* d_zi, void* d_y, int64_t y_row_stride,
+                    void* d_zf, void* d_workspace, size_t workspace_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Exact order statistics of a float32 matrix whose ROWS are spread over several GPUs (the

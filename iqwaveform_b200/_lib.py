@@ -14,7 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # IQW_B200_LIB: another build of the same library (kernel experiments, tools/build_variant.sh)
 LIB_PATH = os.environ.get('IQW_B200_LIB') or os.path.join(_HERE, 'libiqw_b200.so')
 
-ABI_VERSION = 12
+ABI_VERSION = 13
 
 # statuses / enums mirrored from include/iqw_b200.h
 IQW_OK = 0
@@ -78,6 +78,14 @@ SIGNATURES = {
     'iqw_pfb_synthesize_workspace_bytes': (_sz, [_i64, _i64, _i32]),
     'iqw_pfb_synthesize_c64': (ctypes.c_int, [_vp, _i64, _i64, _i64, _i64, _i64, _vp, _i32, _i32, _i32, _i64, _i64,
                                               _vp, _i64, _vp, _sz, _vp]),
+    'iqw_sosfilt_geometry': (ctypes.c_int, [_i32, ctypes.POINTER(_i32)]),
+    'iqw_sosfilt_workspace_bytes': (_sz, [_i64, _i64, _i32]),
+    'iqw_sosfilt_carry_workspace_bytes': (_sz, [_i64, _i64, _i32]),
+    'iqw_sosfilt_states_c64': (ctypes.c_int, [_vp, _i64, _i64, _i64, _vp, _i32, _vp, _vp, _vp, _sz, _vp]),
+    'iqw_sosfilt_carry_c64': (ctypes.c_int, [_vp, _i64, _i64, _vp, _i32, _vp, _vp, _sz, _vp]),
+    'iqw_sosfilt_apply_c64': (ctypes.c_int, [_vp, _i64, _i64, _i64, _vp, _i32, _vp, _vp, _vp, _sz, _vp, _i64, _vp,
+                                             _vp]),
+    'iqw_sosfilt_c64': (ctypes.c_int, [_vp, _i64, _i64, _i64, _vp, _i32, _vp, _vp, _vp, _i64, _vp, _vp, _sz, _vp]),
     'iqw_edge_counts_f32': (ctypes.c_int, [_vp, _i64, _i64, _vp, _i32, _i32, _vp, _vp]),
     'iqw_bracket_collect_workspace_bytes': (_sz, [_i64, _i64]),
     'iqw_bracket_collect_f32': (ctypes.c_int, [_vp, _i64, _i64, _i32, _vp, _vp, _vp, _vp, _sz, _vp]),

@@ -404,3 +404,40 @@ def pfb_taps(h: np.ndarray, nfft: int) -> np.ndarray:
     t = t.reshape(P, nfft)
     t[:, 1::2] *= -1
     return t
+
+
+SOSFILT_MAX_SECTIONS = 16
+
+
+def sosfilt_state_space(sos: np.ndarray) -> tuple[np.ndarray, np.ndarray, np.ndarray, float]:
+    """(A, B, C, D) in float64 of the cascade of direct-form II transposed sections `sos` (S, 6), a0 == 1:
+    z[n+1] = A z[n] + B x[n], y[n] = C z[n] + D x[n], with the 2S states (z1_0, z2_0, z1_1, ...) in
+    scipy.signal.sosfilt's zi order.  A is block lower triangular."""
+    sos = np.asarray(sos, np.float64)
+    n = 2 * len(sos)
+    A, B = np.zeros((n, n)), np.zeros(n)
+    cin, din = np.zeros(n), 1.0          # the input of section s as C z + D x
+    for s, (b0, b1, b2, _, a1, a2) in enumerate(sos):
+        i = 2 * s
+        cy = b0 * cin
+        cy[i] += 1.0
+        dy = b0 * din
+        A[i] = b1 * cin - a1 * cy
+        A[i, i + 1] += 1.0
+        B[i] = b1 * din - a1 * dy
+        A[i + 1] = b2 * cin - a2 * cy
+        B[i + 1] = b2 * din - a2 * dy
+        cin, din = cy, dy
+    return A, B, cin, din
+
+
+def sosfilt_powers(sos: np.ndarray, L: int, G: int, H: int) -> np.ndarray:
+    """float64 (3, 2S, 2S): A^L, A^(L*G), A^(L*G*H) of sosfilt_state_space(sos), by repeated squaring (L, G and H
+    are powers of two) -- the d_powers of the iqw_sosfilt_* entry points"""
+    A = sosfilt_state_space(sos)[0]
+    out = []
+    for steps in (L, G, H):
+        for _ in range(steps.bit_length() - 1):
+            A = A @ A
+        out.append(A)
+    return np.stack(out)

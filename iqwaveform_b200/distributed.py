@@ -18,6 +18,9 @@ The path shards without any collective on the data path, with one exception (the
   [f0, f1) and reads [f0*hop, (f1 - 1)*hop + L), a halo of L - hop samples
 * pfb_synthesize outputs are independent         -> `pfb_synth_shard` (pfb_synthesize): rank r owns outputs
   [o0, o1) and reads the frames that cover them, a halo of about Lg / hop - 1 frames
+* sosfilt is recursive                        -> `sosfilt_shard` (sosfilt): rank r owns the samples of whole
+  groups of kernel 10 and reads no halo; instead the ranks all_gather the zero-state final state of every
+  group, and each folds the whole list into the start states of its own groups (`sosfilt_time_sharded`)
 * exact quantiles of ONE capture split in time -> `persistence_spectrum_time_sharded`: the only
   real exchange step of the path -- per-bin digit counts of a radix select are all_reduced
   (`select_order_statistics`; kernels in csrc/iqw_rowsplit.cu)
@@ -42,7 +45,8 @@ __all__ = ['channel_shard', 'frame_shard', 'bin_shard', 'gather_rows', 'persiste
            'persistence_spectrum_time_sharded', 'select_order_statistics', 'CudaShardOps', 'ThreadGroup',
            'bind_to_gpu_numa_node', 'spectrogram_time_sharded', 'iq_to_bin_power_sharded', 'upfirdn_shard',
            'upfirdn_time_sharded', 'oaconvolve_shard', 'oaconvolve_time_sharded', 'pfb_shard',
-           'pfb_channelize_time_sharded', 'pfb_synth_shard', 'pfb_synthesize_time_sharded']
+           'pfb_channelize_time_sharded', 'pfb_synth_shard', 'pfb_synthesize_time_sharded', 'sosfilt_shard',
+           'SosfiltShardOps', 'sosfilt_time_sharded']
 
 
 def _split(n: int, world: int, rank: int) -> tuple[int, int]:
@@ -737,3 +741,130 @@ def pfb_synthesize_time_sharded(y_halo, g, hop=None, *, n_frames: int, group=Non
                          compute, _on_device(fourier._pfb_synth_device,
                                              'pfb_synthesize: only complex64 frames are built'),
                          group=group, gather=gather, ndim=2, unit='frames')
+
+
+def sosfilt_shard(n_samples: int, n_sections: int, world: int, rank: int) -> OutputShard:
+    """time-axis shard of sosfilt for a capture of n_samples samples and n_sections sections: kernel 10's groups
+    of L*G samples (anchored at sample 0) are split evenly, so every boundary but the capture's end falls on a
+    multiple of L*G.  There is no halo: the samples read are the samples owned."""
+    from . import fourier
+    L, G, _ = fourier._sosfilt_geometry(n_sections)
+    span = L * G
+    g0, g1 = _split(-(-n_samples // span), world, rank)
+    s0, s1 = min(g0 * span, n_samples), min(g1 * span, n_samples)
+    return OutputShard(s0, s1, s0, s1, n_samples)
+
+
+class SosfiltShardOps:
+    """the per-rank device steps of `sosfilt_time_sharded`, through the C-ABI entry points that iqw_sosfilt_c64
+    itself runs, so that the shards reproduce one call bit for bit.  One instance serves one shard: `states`
+    keeps the chunk states in a workspace that `apply` reads.  (The CPU tests substitute a numpy stand-in with
+    the same three methods.)"""
+
+    def __init__(self):
+        self._ws = None
+
+    @staticmethod
+    def _rows(x):
+        from . import _arrays
+        xd, _ = _arrays.to_device(x)
+        if xd.dtype != torch.complex64:
+            raise NotImplementedError(f'sosfilt: only complex64 x is built (got {xd.dtype})')
+        return xd.reshape(1, -1).contiguous()
+
+    def states(self, x, sos32) -> torch.Tensor:
+        """(n_groups, 2S) complex128: the zero-state final state of each group of the shard"""
+        import ctypes
+        from . import _lib, fourier
+        x2 = self._rows(x)
+        S, N = len(sos32), x2.shape[1]
+        L, G, _ = fourier._sosfilt_geometry(S)
+        g = torch.empty((-(-N // (L * G)), 2 * S), dtype=torch.complex128, device=x2.device)
+        ws_bytes = _lib.lib.iqw_sosfilt_workspace_bytes(1, N, S)
+        self._ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x2.device)
+        _lib.check(_lib.lib.iqw_sosfilt_states_c64(
+            ctypes.c_void_p(x2.data_ptr()), 1, N, N, sos32.ctypes.data_as(ctypes.c_void_p), S,
+            ctypes.c_void_p(fourier._sosfilt_powers(sos32, x2.device).data_ptr()), ctypes.c_void_p(g.data_ptr()),
+            ctypes.c_void_p(self._ws.data_ptr()), ws_bytes, fourier._stream_ptr(x2.device)))
+        return g
+
+    def carry(self, g: torch.Tensor, sos32, zi: torch.Tensor | None) -> torch.Tensor:
+        """the group states of the whole capture (n_groups, 2S) -> the start state of each group, from zi (2S,)"""
+        import ctypes
+        from . import _lib, fourier
+        S = len(sos32)
+        g = g.to(torch.complex128).contiguous().clone()
+        if zi is not None:
+            zi = zi.to(g.device).to(torch.complex64).contiguous()
+        ws_bytes = _lib.lib.iqw_sosfilt_carry_workspace_bytes(1, g.shape[0], S)
+        ws = torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=g.device)
+        _lib.check(_lib.lib.iqw_sosfilt_carry_c64(
+            ctypes.c_void_p(g.data_ptr()), 1, g.shape[0], ctypes.c_void_p(zi.data_ptr() if zi is not None else None),
+            S, ctypes.c_void_p(fourier._sosfilt_powers(sos32, g.device).data_ptr()), ctypes.c_void_p(ws.data_ptr()),
+            ws_bytes, fourier._stream_ptr(g.device)))
+        return g
+
+    def apply(self, x, sos32, s: torch.Tensor, want_zf: bool):
+        """the shard's output from the start states s (n_groups, 2S) of its groups -> (y, zf (2S,) or None)"""
+        import ctypes
+        from . import _lib, fourier
+        x2 = self._rows(x)
+        S, N = len(sos32), x2.shape[1]
+        s = s.to(x2.device).to(torch.complex128).contiguous()
+        y = torch.empty_like(x2)
+        zf = torch.zeros(2 * S, dtype=torch.complex64, device=x2.device) if want_zf else None
+        if N:
+            _lib.check(_lib.lib.iqw_sosfilt_apply_c64(
+                ctypes.c_void_p(x2.data_ptr()), 1, N, N, sos32.ctypes.data_as(ctypes.c_void_p), S,
+                ctypes.c_void_p(fourier._sosfilt_powers(sos32, x2.device).data_ptr()), ctypes.c_void_p(s.data_ptr()),
+                ctypes.c_void_p(self._ws.data_ptr()), self._ws.numel(), ctypes.c_void_p(y.data_ptr()), N,
+                ctypes.c_void_p(zf.data_ptr() if zf is not None else None), fourier._stream_ptr(x2.device)))
+        return y[0], zf
+
+
+def sosfilt_time_sharded(x_local, sos, *, n_samples: int, zi=None, group=None, compute=None, gather: bool = False):
+    """time-sharded sosfilt(sos, x) of a 1-D complex64 capture x of `n_samples` samples: `x_local` holds this
+    rank's samples [shard.sample0, shard.sample1) of `sosfilt_shard`.  Each rank runs the states pass on its
+    samples; one all_gather shares every group's zero-state final state; every rank folds the whole list in the
+    order of one call (a small float64 computation) and filters its own samples from the start states of its
+    groups.  Returns this rank's outputs or, with gather=True, all outputs on every rank -- and with `zi` (shape
+    (n_sections, 2)) the pair (y, zf), zf the final state of the whole capture on every rank.  The concatenation
+    is bitwise the single-GPU `sosfilt`.  `compute` is an object with the methods of `SosfiltShardOps`
+    (default: a new `SosfiltShardOps`)."""
+    from . import fourier
+    sos32 = fourier._sosfilt_sos(sos)
+    S = len(sos32)
+    zi_t = None
+    if zi is not None:
+        zi_t = torch.as_tensor(fourier._as_operand(zi))
+        if tuple(zi_t.shape) != (S, 2):
+            raise ValueError(f'Invalid zi shape. With axis=-1, an input with shape {(n_samples,)!r}, and an sos '
+                             f'array with {S} sections, zi must have shape {(S, 2)!r}, got {tuple(zi_t.shape)!r}.')
+        zi_t = zi_t.to(torch.complex64).reshape(2 * S)
+    world, rank = _world(group)
+    L, G, _ = fourier._sosfilt_geometry(S)
+    span = L * G
+    groups = [-(-(sh.sample1 - sh.sample0) // span) for sh in (sosfilt_shard(n_samples, S, world, r)
+                                                                 for r in range(world))]
+    last = max([r for r in range(world) if groups[r] > 0], default=world - 1)
+    zf = []
+
+    def run(ops, sh):
+        g_local = ops.states(x_local, sos32)
+        g_all = torch.view_as_complex(gather_rows(torch.view_as_real(g_local.contiguous()), groups, 0, group)
+                                      .contiguous())
+        first = sum(groups[:rank])
+        s = ops.carry(g_all, sos32, zi_t)[first:first + groups[rank]]
+        y, f = ops.apply(x_local, sos32, s, want_zf=zi_t is not None and rank == last)
+        if zi_t is not None:
+            if n_samples == 0:
+                f = zi_t
+            elif rank != last:
+                f = torch.zeros(2 * S, dtype=torch.complex64, device=y.device)
+            f = torch.view_as_real(f.to(y.device).reshape(1, 2 * S))
+            zf.append(torch.view_as_complex(gather_rows(f, None, 0, group)[last].contiguous()).reshape(S, 2))
+        return y
+
+    y = _time_sharded(x_local, lambda w, r: sosfilt_shard(n_samples, S, w, r), run, compute, SosfiltShardOps(),
+                      group=group, gather=gather)
+    return y if zi is None else (y, zf[0])

@@ -884,6 +884,141 @@ def pfb_synthesize(y, g, hop=None, axis=-2):
     return res.give_back(_arrays.restore_layout(x, lead, trail, 1))
 
 
+_SOSFILT_POWERS: dict = {}
+_SOSFILT_POWERS_LOCK = threading.Lock()
+
+
+def _sosfilt_geometry(n_sections: int) -> tuple[int, int, int]:
+    """(L, G, H) of kernel 10 for n_sections sections: samples per chunk, chunks per group, groups per carry
+    block"""
+    out = (ctypes.c_int32 * 3)()
+    _lib.check(_lib.lib.iqw_sosfilt_geometry(n_sections, out))
+    return out[0], out[1], out[2]
+
+
+def _sosfilt_sos(sos) -> np.ndarray:
+    """scipy.signal.sosfilt's checks of `sos` (ValueError) and what is not built here (NotImplementedError);
+    returns the float32 (n_sections, 6) coefficients"""
+    if isinstance(sos, torch.Tensor):
+        sos = sos.detach().cpu().numpy()
+    sos = np.asarray(sos)
+    if sos.ndim < 2:
+        sos = sos.reshape((1,) * (2 - sos.ndim) + sos.shape)
+    if sos.ndim != 2:
+        raise ValueError('sos array must be 2D')
+    if sos.shape[1] != 6:
+        raise ValueError('sos array must be shape (n_sections, 6)')
+    if not np.all(sos[:, 3] == 1):
+        raise ValueError('sos[:, 3] should be all ones')
+    if np.iscomplexobj(sos):
+        raise NotImplementedError('sosfilt: only real coefficients are built')
+    if sos.dtype.kind not in 'biuf':
+        raise NotImplementedError(f"sosfilt: input type '{sos.dtype}' not supported")
+    if not 1 <= sos.shape[0] <= _plan.SOSFILT_MAX_SECTIONS:
+        raise NotImplementedError(f'sosfilt: {sos.shape[0]} sections (1..{_plan.SOSFILT_MAX_SECTIONS} are built)')
+    sos = np.ascontiguousarray(sos, dtype=np.float32)   # the C entry points read it row by row
+    # largest pole modulus of each section z^2 + a1 z + a2, in closed form so that poles on the unit circle
+    # (integrators, double poles at 1) come out at 1 within a few ulp of float64
+    a1, a2 = sos[:, 4].astype(np.float64), sos[:, 5].astype(np.float64)
+    disc = a1 * a1 - 4 * a2
+    radius = np.where(disc < 0, np.sqrt(np.abs(a2)), (np.abs(a1) + np.sqrt(np.maximum(disc, 0))) / 2)
+    if np.any(radius > 1 + 8 * np.finfo(np.float64).eps) or not np.all(np.isfinite(sos)):
+        s = int(np.argmax(radius))
+        raise NotImplementedError(f'sosfilt: section {s} is unstable (a pole of modulus {radius[s]:.9g} > 1): the '
+                                  f'carry between chunks raises the state matrix to large powers')
+    return sos
+
+
+def _sosfilt_powers(sos32: np.ndarray, device) -> torch.Tensor:
+    """the float64 (3, 2S, 2S) powers of the state matrix on `device`, cached per coefficients and device"""
+    key = (sos32.tobytes(), str(device))
+    with _SOSFILT_POWERS_LOCK:
+        p = _SOSFILT_POWERS.get(key)
+        if p is None:
+            if len(_SOSFILT_POWERS) >= 64:
+                _SOSFILT_POWERS.clear()
+            p = torch.from_numpy(_plan.sosfilt_powers(sos32, *_sosfilt_geometry(len(sos32)))).to(device)
+            _SOSFILT_POWERS[key] = p
+    return p
+
+
+def _sosfilt_device(x2: torch.Tensor, sos32: np.ndarray, zi2: torch.Tensor | None = None,
+                    want_zf: bool = False) -> tuple[torch.Tensor, torch.Tensor | None]:
+    """(C, N) complex64 device rows -> (y (C, N), zf (C, 2S) or None), from start states zi2 (C, 2S) complex64
+    (None: zero).  The kernels read unit-stride rows: any other layout is copied first."""
+    x2 = _arrays.unit_stride_rows(x2)
+    C, N = x2.shape
+    S = len(sos32)
+    y = torch.empty((C, N), dtype=torch.complex64, device=x2.device)
+    zf = torch.empty((C, 2 * S), dtype=torch.complex64, device=x2.device) if want_zf else None
+    if C == 0:
+        return y, zf
+    powers = _sosfilt_powers(sos32, x2.device)
+    ws_bytes = _lib.lib.iqw_sosfilt_workspace_bytes(C, N, S)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x2.device)
+    _lib.check(_lib.lib.iqw_sosfilt_c64(
+        ctypes.c_void_p(x2.data_ptr()), C, N, x2.stride(0) if C > 1 else N, sos32.ctypes.data_as(ctypes.c_void_p), S,
+        ctypes.c_void_p(powers.data_ptr()), ctypes.c_void_p(zi2.data_ptr() if zi2 is not None else None),
+        ctypes.c_void_p(y.data_ptr()), N, ctypes.c_void_p(zf.data_ptr() if zf is not None else None),
+        ctypes.c_void_p(ws.data_ptr()), ws_bytes, _stream_ptr(x2.device)))
+    return y, zf
+
+
+def sosfilt(sos, x, axis=-1, zi=None):
+    """IIR filter `x` along `axis` with the cascade of second-order sections `sos`, each in direct form II
+    transposed: scipy.signal.sosfilt's arguments, checks and result.  With `zi` (scipy's shape (n_sections, ...,
+    2, ...), the 2 at position axis + 1) the start states of the sections, returns (y, zf), zf the final states in
+    zi's shape: filtering a long capture piece by piece, passing each zf on as the next zi, gives the result of
+    one call within the bound below.
+
+    Differences from scipy: the arithmetic is float32.  `sos` (n_sections, 6), real, on the host or the device,
+    is rounded once to float32, and the results are always complex64 -- scipy returns complex128 for float64
+    coefficients.  `x` must be complex64 (numpy, CPU or CUDA torch; y and zf come back as the same kind).  An
+    empty time axis gives an empty y and zf = zi, where scipy fails.  Not built (NotImplementedError): complex
+    coefficients, more than 16 sections, an unstable section (a float32-rounded pole outside the unit circle;
+    poles on it are accepted), and signals of another dtype.
+
+    Kernel 10 cuts each row into chunks anchored at sample 0, filters every chunk from a zero state, carries the
+    states across chunks in float64 through powers of the cascade's state matrix, and filters every chunk again
+    from its carried state (DESIGN.md "Kernel 10").  Every output is the fp32 recursion from the complex64
+    rounding of its chunk's start state, so each row's result depends on that row alone, bit for bit.  Per row,
+    max |y - y64| stays within a small multiple of what scipy's own complex64 sosfilt reaches against float64
+    (DESIGN.md section 7)."""
+    sos32 = _sosfilt_sos(sos)
+    S = len(sos32)
+    dtype = getattr(x, 'dtype', None)
+    if dtype not in (np.complex64, torch.complex64):
+        raise NotImplementedError(f'sosfilt: only complex64 x is built (got {dtype})')
+    shape = tuple(x.shape)
+    ax = axis + len(shape) if axis < 0 else axis
+    if not 0 <= ax < len(shape):
+        raise ValueError(f'axis {axis} exceeds the number of dimensions')
+    zi_shape = (S,) + shape[:ax] + (2,) + shape[ax + 1:]
+    if zi is not None:
+        zi = _as_operand(zi)
+        if tuple(zi.shape) != zi_shape:
+            raise ValueError(f'Invalid zi shape. With axis={axis!r}, an input with shape {shape!r}, and an sos '
+                             f'array with {S} sections, zi must have shape {zi_shape!r}, got {tuple(zi.shape)!r}.')
+    xd, res = _arrays.to_device(x)
+    zt = None
+    if zi is not None:
+        zt = zi if isinstance(zi, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(zi))
+        zt = zt.to(xd.device).to(torch.complex64)
+    if shape[ax] == 0:
+        y = res.give_back(torch.empty(shape, dtype=torch.complex64, device=xd.device))
+        return y if zi is None else (y, res.give_back(zt.contiguous()))
+    x2, lead, trail = _arrays.as_channels(xd, ax)
+    zi2 = None
+    if zt is not None:
+        zi2 = zt.movedim((0, ax + 1), (-2, -1)).reshape(-1, 2 * S).contiguous()
+    y, zf = _sosfilt_device(x2, sos32, zi2, want_zf=zi is not None)
+    y = res.give_back(_arrays.restore_layout(y, lead, trail, 1))
+    if zi is None:
+        return y
+    zf = zf.reshape(lead + trail + (S, 2)).movedim((-2, -1), (0, ax + 1))
+    return y, res.give_back(zf.contiguous())
+
+
 def _python_slice(n: int, start: int, stop_from_end: int) -> tuple[int, int]:
     """bounds of range(n)[start:-stop_from_end] -- including python's [a:-0] == [a:0] (empty)"""
     lo, hi, _ = slice(start, -stop_from_end).indices(n)
